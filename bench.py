@@ -5,6 +5,7 @@
     python bench.py --impl reference ...     # the CPU oracle port on the host cores
     torchrun ... bench.py --gpus N ...       # one rank per GPU: the workload's videos are sharded over
                                              # the ranks in contiguous blocks (strong scaling)
+    python bench.py --dump-outputs DIR ...   # also write the last timed step's outputs as DIR/<name>.npy
 
 The headline workload is BASELINE.json configs[2]: 256 videos x 8 tracks x 120 frames, 180-angle grid —
 the configuration the metric (track-frames x angles / s at 1/2/4/8 B200) is quoted on; it fits one GPU
@@ -43,6 +44,41 @@ UNIT = "track-frame*angle IoU evaluations/s"
 # the clip both arms are quoted on beside their own samples: the reference arm times the CPU port on it,
 # the GPU arm's e2e also runs it through the public API (`e2e.reference_sample`)
 REF_SAMPLE = (1, 40)            # (tracks, frames) of the workload's clip shape and grids
+# --dump-outputs: bytes of all files together; the device pass gets 3/4, the e2e leg 1/4
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_SEED = 2020
+NPY_HEADER = 128                # bytes of a .npy header of these small-rank arrays
+
+
+def dump_arrays(arrays, budget, seed=DUMP_SEED):
+    """name -> tensor  ->  name -> float32 / float64 numpy array, all of them together within ``budget`` bytes.
+    Integer arrays become float64 (exact for 32-bit values); floating arrays keep float32 / float64.  An array
+    larger than its share of the budget is replaced by a seeded sample of its rows (leading dimension) whose
+    sorted indices are stored as ``<name>_rows``; the sample depends only on the shape, so two runs with the same
+    arguments dump the same rows.  Each file is counted with NPY_HEADER bytes of header."""
+    out = {}
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(items):
+        share = budget // (len(items) - i) - NPY_HEADER
+        t = t.detach()
+        dtype = torch.float32 if t.dtype in (torch.float16, torch.bfloat16, torch.float32) else torch.float64
+        n = t.shape[0] if t.dim() else 1
+        row = (t[0].numel() if t.dim() and n else 1) * (4 if dtype == torch.float32 else 8)
+        if n * row > share:
+            k = min(n, max(1, (share - NPY_HEADER) // (row + 8)))
+            rows = np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+            out[name + "_rows"] = rows.astype(np.float64)
+            budget -= out[name + "_rows"].nbytes + NPY_HEADER
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        out[name] = t.to(dtype).cpu().numpy()
+        budget -= out[name].nbytes + NPY_HEADER
+    return out
+
+
+def write_dump(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def _peaks():
@@ -224,10 +260,12 @@ def _committed(name, wl_name, kernel_key):
     return {"value": v, "source": f"committed ncu capture, profiles/{name}.json ({d.get('_source', '')})"}
 
 
-def measure_pass(wl, video_ids, steps, warmup, dev, rank, world, dist, sample_clocks=True, gather=True, streams=1):
+def measure_pass(wl, video_ids, steps, warmup, dev, rank, world, dist, sample_clocks=True, gather=True, streams=1,
+                 dump=None):
     """Device-resident scoring passes over this rank's videos of the workload: K timed steps with CUDA
     events on the launching stream -> dict(value, ms, roofline, ...).  ``value`` is the whole job: the units
-    of all ranks over the slowest rank's step time."""
+    of all ranks over the slowest rank's step time.  ``dump`` (a dict) receives the PassResult of the last
+    timed step as ``pass_*`` arrays (dump_arrays)."""
     from articulation3d_b200 import engine, workloads
 
     inp = workloads.build_pass(wl, seed0=2020, device=dev, video_ids=video_ids)
@@ -314,7 +352,7 @@ def measure_pass(wl, video_ids, steps, warmup, dev, rank, world, dist, sample_cl
     for lane in lanes:
         lane.wait_event(t_begin)
     for k in range(steps):
-        one_step(events[k])
+        last = one_step(events[k])
     for lane in lanes:                                  # join: the timed region ends when every lane has drained
         done = torch.cuda.Event()
         done.record(lane)
@@ -330,6 +368,11 @@ def measure_pass(wl, video_ids, steps, warmup, dev, rank, world, dist, sample_cl
     torch.cuda.synchronize()
     wall, region1 = time.perf_counter() - wall0, time.time()
     clocks = sampler.stop(region0, region1) if sampler else None
+    if dump is not None:                                # before the split steps below overwrite the workspace
+        dump.update(dump_arrays({"pass_" + f: getattr(last, f) for f in (
+            "best_cand", "best_inter", "best_union", "best_iou", "proj_bits", "proj_popc", "proj_bbox")},
+            DUMP_BYTES * 3 // 4))
+    del last                                            # views of the workspace, released with it below
     # the timed K steps: one device interval from the first launch to the last lane / gather draining
     # (with one lane and an L2 flush between steps: the sum of the per-step intervals, which leave the flush out)
     if flush is not None:
@@ -422,9 +465,12 @@ def gpu_arm(args, wl):
         dist.init_process_group("nccl", device_id=dev)
 
     mine = list(a3d_dist.shard_range(wl.videos, rank, world))
-    m = measure_pass(wl, mine, args.steps, args.warmup, dev, rank, world, dist, streams=args.streams)
+    dump = {} if args.dump_outputs and rank == 0 else None
+    m = measure_pass(wl, mine, args.steps, args.warmup, dev, rank, world, dist, streams=args.streams, dump=dump)
     # ---- e2e through the public API with host buffers, sharded like the device-resident pass -----
-    e2e = _e2e(wl, dev, rank, world, dist, steps=max(1, min(args.steps, 5)), videos_per_rank=args.e2e_videos)
+    e2e = _e2e(wl, dev, rank, world, dist, steps=args.steps, videos_per_rank=args.e2e_videos, dump=dump)
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
 
     line = None
     if rank == 0:
@@ -432,7 +478,7 @@ def gpu_arm(args, wl):
         if world == 1 and args.extras:
             # configs[1] (one video, 4 tracks x 60 frames, 90 candidates): a 57 us launch-latency case
             wc = workloads.WORKLOADS["c2"]
-            mc = measure_pass(wc, [0], max(3, min(args.steps, 20)), 3, dev, 0, 1, None, sample_clocks=False)
+            mc = measure_pass(wc, [0], args.steps, 3, dev, 0, 1, None, sample_clocks=False)
             extras["c2"] = {"workload": wc.description, "value": mc["value"], "unit": UNIT,
                             "ms_per_step": mc["ms_per_step"], "units_per_step": mc["units_per_step"], "l2": mc["l2"],
                             "roofline": mc["roofline"]}
@@ -482,7 +528,7 @@ def _pack_stream(dev, n_masks=1024, H=480, W=640, iters=5):
     alone with CUDA events; input (1.26 GB) exceeds L2.  Reported against the measured HBM peak."""
     from articulation3d_b200 import _lib
     lib = _lib.load()
-    src = (torch.rand(n_masks, H, W, device=dev) > 0.7).float()
+    src = (torch.rand(n_masks, H, W, device=dev, generator=torch.Generator(dev).manual_seed(2020)) > 0.7).float()
     pitch = _lib.pitch_words(W)
     bits = torch.empty(n_masks, H, pitch, dtype=torch.int32, device=dev)
     stream = torch.cuda.current_stream().cuda_stream
@@ -554,10 +600,12 @@ def _host_clip(wl, seed, dev, tracks=None, frames=None, pin=True):
     return preds, cfg
 
 
-def _e2e(wl, dev, rank, world, dist, steps, videos_per_rank):
+def _e2e(wl, dev, rank, world, dist, steps, videos_per_rank, dump=None):
     """Public API, host buffers: ``videos_per_rank`` clips of the workload's shape per rank (fp32 masks in
     pinned host memory) -> dist.optimize_videos_sharded (track_planes, H2D, packing, every device pass, D2H,
-    write-back, record gather).  Timed with the wall clock between barriers, max over ranks."""
+    write-back, record gather).  Timed with the wall clock between barriers, max over ranks.  ``dump`` (a dict)
+    receives what the last timed step returned as ``e2e_*`` arrays: this rank's output instances of all frames
+    in video order (scores, planes, axes) and the gathered frame / track records."""
     from articulation3d_b200 import dist as a3d_dist
     from articulation3d_b200 import opt_utils
 
@@ -592,29 +640,38 @@ def _e2e(wl, dev, rank, world, dist, steps, videos_per_rank):
         outs, ids, fr, tr = a3d_dist.optimize_videos_sharded(vids, seeds, cfg=cfg, device=dev, optimize_fn=fn)
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
-        return dt, stats, fr, tr
+        return dt, stats, fr, tr, outs
 
     per_rank = []
 
     def synced_run():
         if dist:
             dist.barrier()
-        dt, st, fr, tr = run()
+        dt, st, fr, tr, outs = run()
         if dist:
             t = torch.zeros(world, device=dev, dtype=torch.float64)
             t[rank] = dt
             dist.all_reduce(t)
             per_rank.append([round(1e3 * float(x), 1) for x in t.tolist()])
             dt = float(t.max().item())
-        return dt, st, fr, tr
+        return dt, st, fr, tr, outs
 
     synced_run()
     restore()
     secs, units, h2d, d2h, passes, sched = 0.0, 0, 0, 0, 0, ""
     n_frame_rec = n_track_rec = 0
     each = []
-    for _ in range(steps):
-        dt, st, fr, tr = synced_run()
+    for k in range(steps):
+        dt, st, fr, tr, outs = synced_run()
+        if dump is not None and k == steps - 1:
+            frames = [p for preds in outs for p in preds]
+            dump.update(dump_arrays({
+                "e2e_scores": torch.from_numpy(np.concatenate([np.asarray(p.scores, dtype=np.float64).reshape(-1)
+                                                               for p in frames])),
+                "e2e_pred_planes": torch.cat([p.pred_planes for p in frames]),
+                "e2e_pred_rot_axis": torch.cat([p.pred_rot_axis for p in frames]),
+                "e2e_pred_tran_axis": torch.cat([p.pred_tran_axis for p in frames]),
+                "e2e_frame_records": fr, "e2e_track_records": tr}, DUMP_BYTES // 4))
         secs += dt
         each.append(round(1e3 * dt, 2))
         u = torch.tensor([st.units_visited, st.h2d_bytes, st.d2h_bytes], device=dev, dtype=torch.int64)
@@ -697,7 +754,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", dest="extras", action="store_false",
                     help="skip the extra single-video (c2) pass and the pack stream reported under 'extras'")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32 / float64, at most "
+                         f"{DUMP_BYTES // 10 ** 6} MB in all, seeded row samples of larger arrays): pass_* = the "
+                         "device pass's PassResult, e2e_* = what the public API returned (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     from articulation3d_b200 import workloads
     wl = workloads.WORKLOADS[args.workload]
     if args.impl == "reference":

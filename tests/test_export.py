@@ -144,20 +144,3 @@ def test_export_equals_reference_fixture(name, tmp_path, golden_dir):
     assert sorted(got) == sorted(want)
     for k in want:
         assert got[k] == want[k], f"{k} differs from the reference's file"
-
-
-@pytest.mark.slow
-@pytest.mark.parametrize("seed,frame_id,axis_dir", [(11, 2, "l"), (12, 9, "r")])
-def test_export_equals_live_reference(seed, frame_id, axis_dir, tmp_path):
-    """The same comparison against the reference executed now (only where /root/reference exists)."""
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip("reference sources not on this box")
-    from oracle import ref_export
-    from oracle.gen_golden import export_digest
-    preds, _ = synth.make_video(seed, 2, 12, kinds=[0, 1])
-    image = np.random.RandomState(seed).randint(0, 256, size=(480, 640, 3)).astype(np.uint8)
-    rp = synth.clone_preds(preds, ref_shim.Instances, ref_shim.Boxes)
-    ref_dir = ref_export.run_reference_export(rp, [image] * len(preds), frame_id, str(tmp_path / "ref"), axis_dir=axis_dir)
-    obj = export.save_obj_model(str(tmp_path / "own"), preds, frame_id, image=image, axis_dir=axis_dir)
-    assert export_digest(os.path.dirname(obj)) == export_digest(ref_dir)

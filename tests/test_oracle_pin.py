@@ -1,8 +1,6 @@
-"""Pins the CPU oracle (oracle/restated.py):
-
-* against the committed fixtures in tests/golden/ — outputs of the UNMODIFIED
-  reference run under oracle/ref_shim.py in the build container;
-* where /root/reference is present, against the live reference on extra seeds.
+"""Pins the CPU oracle (oracle/restated.py) against the committed fixtures in
+tests/golden/ — outputs of the UNMODIFIED reference run under oracle/ref_shim.py
+(oracle/gen_golden.py regenerates them where the reference sources exist).
 """
 import random
 
@@ -10,9 +8,8 @@ import numpy as np
 import pytest
 import torch
 
-from articulation3d_b200 import synth
 from articulation3d_b200.structures import Boxes, Instances
-from oracle import ref_shim, restated
+from oracle import restated
 from tests import golden_util as gu
 
 
@@ -64,22 +61,6 @@ def test_golden_covers_both_outcomes():
             for i in range(int(z[f"{cat}_n"])):
                 seen.add((cat, bool(z[f"{cat}{i}_has_rot"])))
     assert ("rot", True) in seen and ("rot", False) in seen and ("trans", True) in seen
-
-
-@pytest.mark.slow
-@pytest.mark.skipif(not ref_shim.available(), reason="reference sources not on this box")
-@pytest.mark.parametrize("seed,n_tracks,n_frames,drop", [(31, 3, 14, 0.0), (32, 2, 18, 0.1)])
-def test_restated_oracle_matches_live_reference(seed, n_tracks, n_frames, drop, monkeypatch):
-    from oracle.gen_golden import run_reference
-    preds, _ = synth.make_video(seed, n_tracks, n_frames, drop_prob=drop)
-    ref = run_reference(synth.clone_preds(preds, ref_shim.Instances, ref_shim.Boxes), seed)
-    ref["image_size"] = np.array(preds[0].image_size)
-
-    class Z(dict):
-        files = property(lambda self: list(self.keys()))
-
-    planes, out, choices, lin, _ = run_restated(synth.clone_preds(preds), seed, monkeypatch)
-    gu.check_against_golden(Z(ref), planes, out, choices, lin)
 
 
 @pytest.mark.parametrize("name", ["depth_a", "depth_b"])
