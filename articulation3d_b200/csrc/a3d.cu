@@ -612,8 +612,9 @@ __device__ __forceinline__ void splat_job(const Cam& cam, const a3d_job_t& job, 
             }
         }
     };
-    // full rounds: every thread owns one 8-point item and applies all candidates of the tile to it
-    const int nfull = (nitems / kStride) * kStride;
+    // full rounds: every thread owns one 8-point item and applies all candidates of the tile to it; only
+    // items of 8 written points take part, so a last item of fewer points always falls in the tail below
+    const int nfull = ((npts / kProjPX) / kStride) * kStride;
     for (int item = tid; item < nfull; item += kStride) {
         float X[kProjPX], Y[kProjPX], Z[kProjPX];
         load_item(item, X, Y, Z);
@@ -844,8 +845,8 @@ __device__ __forceinline__ void splat_job_filter(const Cam& cam, const a3d_job_t
             if (k < nvalid) C = (cc[k] >= C) ? cc[k] : C;         // +inf propagates (a written C is never NaN)
     };
     // full rounds: every thread owns one 8-point item and applies the candidates of the tile to it, 8 at a
-    // time (the unproven pairs of 8 candidates x 8 points fit one 64-bit mask)
-    const int nfull = (nitems / kStride) * kStride;
+    // time (the unproven pairs of 8 candidates x 8 points fit one 64-bit mask); only items of 8 written points
+    const int nfull = ((npts / kProjPX) / kStride) * kStride;
     for (int item = tid; item < nfull; item += kStride) {
         float xs[kProjPX], ys[kProjPX], C;
         load_item(item, xs, ys, C, kProjPX);
@@ -2748,9 +2749,13 @@ static int score_impl(int H, int W, const a3d_job_t* jobs, int n_jobs, int max_t
         const int tt_tiles = (max_tgt + kScoreTT - 1) / kScoreTT, ct_tiles = (max_cand + 4 * wc - 1) / (4 * wc);
         const long long nblocks = (long long)n_jobs * tt_tiles * ct_tiles;
         if (nblocks > 0x7fffffffLL) return fail(A3D_ELIMIT, "a3d_score: too many (job, tile) blocks");
+        // A3D_SCORE_ADDR=wide forces 64-bit mask addressing, which only pools or candidate buffers of
+        // 2^32 words and more need, so that it can be checked on small inputs
+        const char* env_addr = getenv("A3D_SCORE_ADDR");
         const unsigned long long words = (unsigned long long)H * pitch;
         const bool narrow = (unsigned long long)n_pool_masks * words < (1ull << 32) &&
-                            (unsigned long long)n_cand_total * words < (1ull << 32);
+                            (unsigned long long)n_cand_total * words < (1ull << 32) &&
+                            !(env_addr && !strcmp(env_addr, "wide"));
 #define A3D_LAUNCH_SCORE(N, WC)                                                                                    \
     A3D_CUDA_TRY(launch(k_score<N, WC, WC == 2>, dim3((unsigned)nblocks), dim3(256), 0, s, pdl, jobs, H, pitch, tt_tiles, \
                         ct_tiles, tgt_bits, tgt_popc, tgt_bbox, tgt_index, proj_bits, proj_popc, proj_bbox,         \

@@ -393,7 +393,7 @@ class DeviceBatch:
             plan = plan_tiles_native(batch.jobs, max_tile(cfg), plan_sm_count(device))
             if plan[1] is None:
                 plan = (choose_tile(cfg, int(batch.xform.shape[0]), batch.n_jobs, plan_sm_count(device)), None)
-            self._plans[(cfg.height, cfg.width)] = plan
+            self._plans[_plan_key(cfg)] = plan
         tmap = plan[1] if plan is not None and plan[1] is not None else np.zeros((0, 4), np.int32)
         self.n_jobs = batch.n_jobs
         self.n_cand_total = int(batch.xform.shape[0])
@@ -429,11 +429,11 @@ class DeviceBatch:
         self.jobs = dev[oj:oj + nj]
         self.xform = dev[ox:ox + nx].view(torch.float32).view(-1, 12)
         self.tgt_index = dev[ot:ot + nt].view(torch.int32)
-        self._tmap_dev = {(cfg.height, cfg.width): dev[om:om + nm].view(torch.int32).view(-1, 4)} if nm else {}
+        self._tmap_dev = {_plan_key(cfg): dev[om:om + nm].view(torch.int32).view(-1, 4)} if nm else {}
 
     def tile_plan(self, cfg: OptConfig):
         """(tile_cand, device tile map or None) for this camera: planned once, uploaded once."""
-        key = (cfg.height, cfg.width)
+        key = _plan_key(cfg)
         if key not in self._plans:
             if os.environ.get("A3D_TILE_PLAN") == "uniform":
                 self._plans[key] = (choose_tile(cfg, self.n_cand_total, self.n_jobs, plan_sm_count(self.device)), None)
@@ -541,9 +541,15 @@ def _camera_cached(cfg: OptConfig) -> _lib.Camera:
     return cam
 
 
+def _plan_key(cfg: OptConfig):
+    """What the largest projection tile depends on: the image size and the projection schedule."""
+    return cfg.height, cfg.width, os.environ.get("A3D_PROJECT_SCHED")
+
+
 def max_tile(cfg: OptConfig) -> int:
-    """Most candidates one projection CTA holds in shared memory for this image size."""
-    key = (cfg.height, cfg.width)
+    """Most candidates one projection CTA holds in shared memory for this image size and projection schedule
+    (persistent CTAs hold two groups of slots, so A3D_PROJECT_SCHED=persistent halves the limit)."""
+    key = _plan_key(cfg)
     t = _tile_cache.get(key)
     if t is None:
         lib = _lib.load()
