@@ -43,6 +43,7 @@ EXPORTS = (
     "a3d_version", "a3d_last_error_string", "a3d_pitch_words", "a3d_project_max_tile",
     "a3d_pack_masks", "a3d_mask_meta", "a3d_project", "a3d_score", "a3d_pass", "a3d_emit_masks",
     "a3d_rle_to_bits", "a3d_plane_offsets", "a3d_plan_tiles", "a3d_host_quat_to_xform", "a3d_fetch_host_block", "a3d_upload_masks", "a3d_host_rle_counts",
+    "a3d_rle_count_runs", "a3d_bits_to_rle", "a3d_host_rle_strings",
 )
 
 _lib = None
@@ -91,12 +92,18 @@ def load():
     lib.a3d_fetch_host_block.argtypes = [vp, vp, i64, vp]
     lib.a3d_host_rle_counts.restype = C.c_int64
     lib.a3d_host_rle_counts.argtypes = [vp, vp, i64, vp, i64, vp, vp]
+    lib.a3d_host_rle_strings.restype = C.c_int64
+    lib.a3d_host_rle_strings.argtypes = [vp, vp, i64, vp, i64, vp]
     lib.a3d_upload_masks.restype = C.c_int
     lib.a3d_upload_masks.argtypes = [vp, vp, i32, i32, i32, i32, f32, vp, i64, vp, vp, i32, vp]
     lib.a3d_emit_masks.restype = C.c_int
     lib.a3d_emit_masks.argtypes = [vp, vp, i64, i32, i32, i32, vp, vp]
     lib.a3d_rle_to_bits.restype = C.c_int
     lib.a3d_rle_to_bits.argtypes = [vp, vp, i64, i32, i32, vp, vp]
+    lib.a3d_rle_count_runs.restype = C.c_int
+    lib.a3d_rle_count_runs.argtypes = [vp, vp, i64, i32, i32, vp, vp]
+    lib.a3d_bits_to_rle.restype = C.c_int
+    lib.a3d_bits_to_rle.argtypes = [vp, vp, i64, i32, i32, vp, vp, vp]
     lib.a3d_plane_offsets.restype = C.c_int
     lib.a3d_plane_offsets.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp, vp]
     _lib = lib

@@ -2087,6 +2087,153 @@ k_emit(const uint32_t* __restrict__ bits, const int32_t* __restrict__ index, int
     }
 }
 
+// ---------------------------------------------------------------------------
+// bits -> COCO RLE (column-major runs, alternating 0/1, starting with 0s).
+// A run boundary sits at flat position p = x*H + y wherever pixel (y, x) differs from its column-major
+// predecessor: (y-1, x) for y >= 1, (H-1, x-1) for y == 0, a virtual 0 for (0, 0) (a set first pixel opens
+// with an empty 0-run).  As packed words that is the transition row D[y] = R[y] ^ R[y-1], and for row 0
+// D[0] = R[0] ^ (R[H-1] shifted up by one pixel, bit 31 of word j-1 carried into bit 0 of word j, a 0 into
+// pixel 0); only the W valid bits of every row are read or kept.  A mask has popc(D) + 1 runs; the runs are
+// the differences of consecutive boundary positions, with 0 as the first bound and H*W as the last.
+// ---------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t rle_valid(int j, int W) {
+    const int left = W - 32 * j;
+    return left >= 32 ? 0xffffffffu : ((1u << left) - 1u);
+}
+
+// transition word D[y][j] of one packed mask
+__device__ __forceinline__ uint32_t rle_transitions(const uint32_t* __restrict__ b, int H, int W, int pitch, int y, int j) {
+    const uint32_t valid = rle_valid(j, W);
+    const uint32_t r = b[(int64_t)y * pitch + j] & valid;
+    uint32_t prev;
+    if (y > 0) {
+        prev = b[(int64_t)(y - 1) * pitch + j] & valid;
+    } else {
+        const uint32_t* last = b + (int64_t)(H - 1) * pitch;
+        prev = ((last[j] & valid) << 1) | (j > 0 ? last[j - 1] >> 31 : 0u);
+    }
+    return (r ^ prev) & valid;
+}
+
+// runs_out[i] = popc(D) + 1 of mask index[i]; one CTA per mask (grid-stride), coalesced over the mask's words
+__global__ void __launch_bounds__(256)
+k_rle_count(const uint32_t* __restrict__ bits, const int32_t* __restrict__ index, int64_t n, int H, int W, int pitch,
+            int64_t* __restrict__ runs_out) {
+    __shared__ int64_t s_sum[8];
+    const int nw = (W + 31) >> 5;
+    const int64_t words = (int64_t)H * nw;
+    for (int64_t i = blockIdx.x; i < n; i += gridDim.x) {
+        const uint32_t* b = bits + (index ? (int64_t)index[i] : i) * H * pitch;
+        int64_t c = 0;
+        for (int64_t w = threadIdx.x; w < words; w += blockDim.x) {
+            const int y = (int)(w / nw), j = (int)(w - (int64_t)y * nw);
+            c += __popc(rle_transitions(b, H, W, pitch, y, j));
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
+        if ((threadIdx.x & 31) == 0) s_sum[threadIdx.x >> 5] = c;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            int64_t t = 1;
+            for (int k = 0; k < 8; ++k) t += s_sum[k];
+            runs_out[i] = t;
+        }
+        __syncthreads();
+    }
+}
+
+// The 32x32 tile of D at word column j, rows y0..y0+31, transposed: lane c gets the transition bits of pixel
+// column 32j + c, bit r = row y0 + r.  One ballot per column; tiles without a transition return 0 at once.
+__device__ __forceinline__ uint32_t rle_tile_column(const uint32_t* __restrict__ b, int H, int W, int pitch, int y0,
+                                                    int j, int lane) {
+    const int y = y0 + lane;
+    const uint32_t d = y < H ? rle_transitions(b, H, W, pitch, y, j) : 0u;
+    if (!__any_sync(0xffffffffu, d != 0u)) return 0u;
+    uint32_t mine = 0;
+#pragma unroll
+    for (int c = 0; c < 32; ++c) {
+        const uint32_t t = __ballot_sync(0xffffffffu, (d >> c) & 1u);
+        if (lane == c) mine = t;
+    }
+    return mine;
+}
+
+// counts_out[begin[i] ..] = runs of mask index[i].  One CTA per mask (grid-stride), one warp per word column;
+// the word columns are taken in groups of 8 (one per warp) so that no per-column state needs shared memory
+// whatever W is.  Per group: pass 1 counts every pixel column's transitions and finds its last one; a scan
+// over lanes, over the group's warps and the carry of the earlier groups gives each lane the rank of its
+// first transition and the position of the transition before it; pass 2 re-walks the column and writes the
+// differences.  The transposed tiles are re-read rather than kept (L1 / L2 hits: a 640x480 mask is 38 KB).
+constexpr int kRleWarps = 8;
+__global__ void __launch_bounds__(kRleWarps * 32)
+k_bits_to_rle(const uint32_t* __restrict__ bits, const int32_t* __restrict__ index, int64_t n, int H, int W,
+              int pitch, const int64_t* __restrict__ begin, uint32_t* __restrict__ counts_out) {
+    __shared__ int64_t s_cnt[kRleWarps];
+    __shared__ int64_t s_last[kRleWarps];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int nw = (W + 31) >> 5;
+    for (int64_t i = blockIdx.x; i < n; i += gridDim.x) {
+        const uint32_t* b = bits + (index ? (int64_t)index[i] : i) * H * pitch;
+        const int64_t out0 = begin[i], n_runs = begin[i + 1] - out0;
+        uint32_t* out = counts_out + out0;
+        int64_t carry_cnt = 0, carry_last = 0;          // transitions of the earlier groups; position of the last
+        for (int g = 0; g < nw; g += kRleWarps) {
+            const int j = g + warp;
+            const int64_t col0 = (int64_t)(32 * j + lane) * H;     // this lane's pixel column starts here
+            // pass 1: transitions of column x and the position of its last one (-1: none)
+            int64_t cnt = 0, last = -1;
+            if (j < nw) {
+                for (int y0 = 0; y0 < H; y0 += 32) {
+                    const uint32_t t = rle_tile_column(b, H, W, pitch, y0, j, lane);
+                    if (t) {
+                        cnt += __popc(t);
+                        last = col0 + y0 + 31 - __clz(t);
+                    }
+                }
+            }
+            // scans over lanes: transitions before this column, last transition before it
+            int64_t incl = cnt, mx = last;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const int64_t a = __shfl_up_sync(0xffffffffu, incl, d);
+                const int64_t m = __shfl_up_sync(0xffffffffu, mx, d);
+                if (lane >= d) { incl += a; mx = m > mx ? m : mx; }
+            }
+            const int64_t excl = incl - cnt;
+            int64_t prev_in_warp = __shfl_up_sync(0xffffffffu, mx, 1);
+            if (lane == 0) prev_in_warp = -1;
+            if (lane == 31) { s_cnt[warp] = incl; s_last[warp] = mx; }
+            __syncthreads();
+            int64_t rank = carry_cnt + excl, prev = carry_last;
+            for (int k = 0; k < warp; ++k) {
+                rank += s_cnt[k];
+                prev = s_last[k] > prev ? s_last[k] : prev;
+            }
+            prev = prev_in_warp > prev ? prev_in_warp : prev;
+            // pass 2 (the whole warp, for its ballots): the runs that end at this column's transitions
+            if (j < nw && __any_sync(0xffffffffu, cnt > 0)) {
+                for (int y0 = 0; y0 < H; y0 += 32) {
+                    uint32_t t = rle_tile_column(b, H, W, pitch, y0, j, lane);
+                    while (t) {
+                        const int r = __ffs(t) - 1;
+                        t &= t - 1;
+                        const int64_t pos = col0 + y0 + r;
+                        if (rank < n_runs - 1) out[rank] = (uint32_t)(pos - prev);
+                        prev = pos;
+                        ++rank;
+                    }
+                }
+            }
+            for (int k = 0; k < kRleWarps; ++k) {
+                carry_cnt += s_cnt[k];
+                carry_last = s_last[k] > carry_last ? s_last[k] : carry_last;
+            }
+            __syncthreads();
+        }
+        if (threadIdx.x == 0 && carry_cnt == n_runs - 1) out[carry_cnt] = (uint32_t)((int64_t)H * W - carry_last);
+    }
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -2290,6 +2437,37 @@ int64_t a3d_host_rle_counts(const uint8_t* chars, const int64_t* begin, int64_t 
     }
     if (count_begin_out) count_begin_out[n] = total;
     return total;
+}
+
+// Run lengths -> COCO compressed strings (the inverse of a3d_host_rle_counts; rle.counts_to_string restated):
+// from the fourth count of a mask on, the count is stored as its difference to the count two places back (signed,
+// 64-bit), each
+// value as 5-bit groups, least significant first, 0x20 = more groups follow, +48; the last group's bit 4 is the
+// sign.
+int64_t a3d_host_rle_strings(const uint32_t* counts, const int64_t* begin, int64_t n, uint8_t* chars_out,
+                             int64_t cap, int64_t* char_begin_out) {
+    if (n < 0 || cap < 0 || (n > 0 && (!counts || !begin)) || (cap > 0 && !chars_out))
+        return fail(A3D_EINVAL, "a3d_host_rle_strings: bad argument");
+    int64_t p = 0;
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t b = begin[i], e = begin[i + 1];
+        if (b < 0 || e < b) return fail(A3D_EINVAL, "a3d_host_rle_strings: mask %lld: bad offsets", (long long)i);
+        if (char_begin_out) char_begin_out[i] = p;
+        for (int64_t k = b; k < e; ++k) {
+            int64_t x = (int64_t)counts[k];
+            if (k - b > 2) x -= (int64_t)counts[k - 2];
+            for (bool more = true; more;) {
+                unsigned c = (unsigned)(x & 0x1f);
+                x >>= 5;                                    // arithmetic: the sign is kept
+                more = (c & 0x10u) ? x != -1 : x != 0;
+                if (more) c |= 0x20u;
+                if (p >= cap) return fail(A3D_EINVAL, "a3d_host_rle_strings: chars_out holds %lld bytes, more are needed", (long long)cap);
+                chars_out[p++] = (uint8_t)(c + 48);
+            }
+        }
+    }
+    if (char_begin_out) char_begin_out[n] = p;
+    return p;
 }
 
 int a3d_plan_tiles(const a3d_job_t* jobs_host, int n_jobs, int tile_max, int sm_count, int32_t* tile_map_out,
@@ -2793,6 +2971,42 @@ int a3d_emit_masks(const uint32_t* bits, const int32_t* index, int64_t n, int H,
         k_emit<unsigned char><<<grid, 256, 0, s>>>(bits, index, H, W, pitch, (unsigned char*)out);
     else
         return fail(A3D_EINVAL, "a3d_emit_masks: unknown dtype %d", out_dtype);
+    A3D_CUDA_TRY(cudaGetLastError());
+    return A3D_OK;
+}
+
+// shape checks shared by the two encoder calls; 1 = nothing to do, 0 = go on, < 0 = error
+static int rle_encode_args(const char* what, const uint32_t* bits, int64_t n, int H, int W, const void* a,
+                           const void* b) {
+    if (n < 0 || H <= 0 || W <= 0) return fail(A3D_EINVAL, "%s: bad shape n=%lld %dx%d", what, (long long)n, H, W);
+    if ((int64_t)H * W > 0x7fffffffLL)
+        return fail(A3D_ELIMIT, "%s: a %dx%d mask has more than 2^31 - 1 pixels", what, H, W);
+    if (n == 0) return 1;
+    if (!bits || !a || !b) return fail(A3D_EINVAL, "%s: null pointer", what);
+    return 0;
+}
+
+static unsigned rle_grid(int64_t n) {
+    const int sms = device_sm_count();
+    const int64_t cap = (int64_t)(sms > 0 ? sms : 1) * 16;
+    return (unsigned)(n < cap ? n : cap);
+}
+
+int a3d_rle_count_runs(const uint32_t* bits, const int32_t* index, int64_t n, int H, int W, int64_t* runs_out,
+                       void* stream) {
+    const int rc = rle_encode_args("a3d_rle_count_runs", bits, n, H, W, runs_out, runs_out);
+    if (rc) return rc < 0 ? rc : A3D_OK;
+    k_rle_count<<<rle_grid(n), 256, 0, (cudaStream_t)stream>>>(bits, index, n, H, W, pitch_words(W), runs_out);
+    A3D_CUDA_TRY(cudaGetLastError());
+    return A3D_OK;
+}
+
+int a3d_bits_to_rle(const uint32_t* bits, const int32_t* index, int64_t n, int H, int W, const int64_t* begin,
+                    uint32_t* counts_out, void* stream) {
+    const int rc = rle_encode_args("a3d_bits_to_rle", bits, n, H, W, begin, counts_out);
+    if (rc) return rc < 0 ? rc : A3D_OK;
+    k_bits_to_rle<<<rle_grid(n), kRleWarps * 32, 0, (cudaStream_t)stream>>>(bits, index, n, H, W, pitch_words(W),
+                                                                             begin, counts_out);
     A3D_CUDA_TRY(cudaGetLastError());
     return A3D_OK;
 }

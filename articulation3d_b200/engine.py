@@ -663,6 +663,41 @@ def emit_masks(bits: torch.Tensor, index: torch.Tensor | None, H: int, W: int,
     return out
 
 
+def bits_to_rle(bits: torch.Tensor, H: int, W: int, index: torch.Tensor | None = None,
+                ws: Workspace | None = None):
+    """COCO run lengths of packed masks ((n, H, pitch) int32 on the device; ``index`` selects masks as in
+    ``emit_masks``), encoded on the device: the run count of every mask, a device scan into ``begin``, one
+    synchronising read of the total, the runs, one D2H copy of runs and ``begin``.  Returns (flat uint32
+    counts, int64 begin[n+1]) on the host; mask i's runs are ``counts[begin[i]:begin[i+1]]``."""
+    lib = _lib.load()
+    _require_cuda(bits, "bits")
+    if bits.dtype != torch.int32 or bits.dim() != 3 or bits.shape[1] != H or bits.shape[2] != _lib.pitch_words(W):
+        raise ValueError(f"bits must be (n, {H}, {_lib.pitch_words(W)}) int32")
+    bits = bits.contiguous()
+    if index is not None:
+        index = index.to(device=bits.device, dtype=torch.int32).contiguous()
+    n = int(index.numel()) if index is not None else int(bits.shape[0])
+    ws = ws or Workspace(bits.device)
+    idx_ptr = index.data_ptr() if index is not None else None
+    with torch.cuda.device(bits.device):
+        stream = _stream_ptr()
+        runs = ws.get("rle_runs", (n,), torch.int64)
+        _lib.check(lib.a3d_rle_count_runs(bits.data_ptr(), idx_ptr, n, H, W, runs.data_ptr(), stream),
+                   "a3d_rle_count_runs")
+        scan = ws.get("rle_scan", (n + 1,), torch.int64)
+        scan[0] = 0
+        torch.cumsum(runs, 0, out=scan[1:])
+        total = int(scan[n])
+        # one block for the single D2H copy: begin [n+1] int64, then the runs as uint32
+        out = ws.get("rle_out", (n + 1 + (total + 1) // 2,), torch.int64)
+        out[:n + 1].copy_(scan)
+        counts = out[n + 1:].view(torch.int32)
+        _lib.check(lib.a3d_bits_to_rle(bits.data_ptr(), idx_ptr, n, H, W, out.data_ptr(), counts.data_ptr(), stream),
+                   "a3d_bits_to_rle")
+        host = out.cpu().numpy()
+    return host[n + 1:].view(np.uint32)[:total], host[:n + 1]
+
+
 def rle_to_pool(rles, H: int, W: int, device) -> MaskPool:
     """COCO RLE dicts -> MaskPool, decoded on the device straight into packed bits
     (no dense mask is ever materialised).  ``rles``: sequence of

@@ -20,21 +20,41 @@ from . import adapter, geometry, rle
 from .config import OptConfig
 
 
-def preds_to_records(preds, video_id: str = "synthetic00_0_0", start_image_id: int = 0):
-    """list[Instances] (dense masks) -> list of reference-format records (RLE masks)."""
+def preds_to_records(preds, video_id: str = "synthetic00_0_0", start_image_id: int = 0, device=None):
+    """list[Instances] (dense masks) -> list of reference-format records (RLE masks).  With a CUDA ``device`` the
+    masks are thresholded (``> 0.5``), packed and encoded there, with the same records as a result."""
+    segs = None
+    if device is not None:
+        segs = iter(_encode_preds_on_device(preds, torch.device(device)))
     records = []
     for t, p in enumerate(preds):
         boxes = p.pred_boxes.tensor.numpy().astype(np.float64)
         inst = []
         for k in range(len(boxes)):
             x0, y0, x1, y1 = boxes[k].tolist()
+            seg = next(segs) if segs is not None else rle.encode(p.pred_masks[k].numpy() > 0.5)
             inst.append({"image_id": start_image_id + t, "category_id": int(p.pred_classes[k]),
                          "bbox": [x0, y0, x1 - x0, y1 - y0], "score": float(p.scores[k]),
-                         "segmentation": rle.encode(p.pred_masks[k].numpy() > 0.5)})
+                         "segmentation": seg})
         records.append({"image_id": start_image_id + t, "file_name": f"{video_id}_{t}.png", "instances": inst,
                         "pred_plane": p.pred_planes.clone(), "pred_rot_axis": p.pred_rot_axis.clone(),
                         "pred_tran_axis": p.pred_tran_axis.clone()})
     return records
+
+
+def _encode_preds_on_device(preds, device) -> list:
+    """RLE dicts of every instance mask of the clip (``pred_masks > 0.5``), frame by frame."""
+    from . import engine
+    n = sum(len(p.pred_masks) for p in preds)
+    if n == 0:
+        return []
+    H, W = preds[0].pred_masks.shape[1:]
+    pool = engine.PoolBuilder(n, H, W, device, thresh=0.5)
+    with torch.cuda.device(device):
+        for p in preds:
+            if len(p.pred_masks):
+                pool.append(p.pred_masks.to(device))
+    return rle.bits_to_rles(pool.bits, H, W)
 
 
 def records_to_preds(records, image_size=None, conf_threshold: float = 0.7, masks: str = "rle"):
@@ -67,9 +87,11 @@ def opt_preds_to_records(opt_preds, records):
     return out
 
 
-def tracks_summary(planes) -> list:
+def tracks_summary(planes, masks: bool = False) -> list:
     """JSON-able fitted results per track: has_rot, std_axis, centre frame, R^2, and the
-    angle-per-frame track (frame, angle index, angle value, inter, union, iou)."""
+    angle-per-frame track (frame, angle index, angle value, inter, union, iou).  ``masks=True`` adds to every
+    angle-track entry its registered mask (``plane['reg_masks']``) as COCO RLE, ``segmentation`` =
+    ``{"size": [H, W], "counts": <ascii str>}``."""
     out = []
     for cat in ("trans", "rot"):
         for ti, plane in enumerate(planes[cat]):
@@ -85,15 +107,32 @@ def tracks_summary(planes) -> list:
                      "iou": None if np.isnan(o) else float(o)}
                     for f, a, v, i, u, o in zip(fit["frames"], fit["angle_id"], fit["angle"], fit["inter"],
                                                 fit["union"], fit["iou"])]
+                if masks:
+                    segs = _reg_mask_rles(plane["reg_masks"])
+                    for e in rec["angle_track"]:
+                        seg = segs[e["frame"]]
+                        e["segmentation"] = {"size": list(seg["size"]), "counts": seg["counts"].decode("ascii")}
             out.append(rec)
     return out
 
 
-def save_results(out_dir: str, video_id: str, opt_records, planes):
+def _reg_mask_rles(reg_masks) -> dict:
+    """frame -> RLE of the registered masks: on the device for the optimiser's packed ``RegMasks``, on the host
+    for a plain mapping of dense masks."""
+    if hasattr(reg_masks, "to_rle"):
+        return reg_masks.to_rle()
+    frames = list(reg_masks.keys())
+    dense = np.stack([np.asarray(reg_masks[f]) for f in frames]) if frames else np.zeros((0, 1, 1), np.float32)
+    return dict(zip(frames, rle.encode_many(dense)))
+
+
+def save_results(out_dir: str, video_id: str, opt_records, planes, masks: bool = False):
+    """``<video_id>_predictions_opt.pth`` (the records) and ``<video_id>_tracks.json`` (``tracks_summary``; with
+    ``masks=True`` it carries the registered masks)."""
     os.makedirs(out_dir, exist_ok=True)
     torch.save(opt_records, os.path.join(out_dir, f"{video_id}_predictions_opt.pth"))
     with open(os.path.join(out_dir, f"{video_id}_tracks.json"), "w") as f:
-        json.dump(tracks_summary(planes), f, indent=1)
+        json.dump(tracks_summary(planes, masks=masks), f, indent=1)
 
 
 def write_obj(path: str, preds, planes, frame: int, cfg: OptConfig | None = None):

@@ -205,6 +205,12 @@ class RegMasks(Mapping):
         """All masks as one (T, H, W) device tensor."""
         return engine.emit_masks(self.packed, None, self._H, self._W, dtype=dtype)
 
+    def to_rle(self) -> dict:
+        """frame -> COCO RLE dict of every mask, encoded on the device from the packed copy in one call (no dense
+        image is made, nothing is cached)."""
+        from . import rle
+        return dict(zip(self._frames, rle.bits_to_rles(self.packed, self._H, self._W)))
+
 
 # ---------------------------------------------------------------------------
 # the host control flow, as a generator of device jobs

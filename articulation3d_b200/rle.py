@@ -101,6 +101,58 @@ def encode(mask: np.ndarray) -> dict:
     return {"size": [h, w], "counts": counts_to_string(runs)}
 
 
+def counts_to_strings(counts, begin) -> list:
+    """Run lengths of many masks (flat uint32 ``counts``, int64 ``begin[n+1]``) -> their compressed strings, written
+    by the library's host helper (``a3d_host_rle_strings``, byte for byte ``counts_to_string``)."""
+    from . import _lib
+    lib = _lib.load()
+    counts = np.ascontiguousarray(counts, dtype=np.uint32)
+    begin = np.ascontiguousarray(begin, dtype=np.int64)
+    n = len(begin) - 1
+    cap = 7 * max(len(counts), 1)                 # a difference of two uint32 counts takes at most 7 characters
+    chars = np.empty(cap, dtype=np.uint8)
+    cbeg = np.zeros(n + 1, dtype=np.int64)
+    _lib.check(lib.a3d_host_rle_strings(counts.ctypes.data, begin.ctypes.data, n, chars.ctypes.data, cap,
+                                        cbeg.ctypes.data), "a3d_host_rle_strings")
+    blob = chars.tobytes()
+    return [blob[cbeg[i]:cbeg[i + 1]] for i in range(n)]
+
+
+def bits_to_rles(bits, H: int, W: int, index=None) -> list:
+    """Packed masks on the device ((n, H, pitch) int32, ``index`` as in ``engine.emit_masks``) -> COCO RLE dicts,
+    encoded on the GPU (``engine.bits_to_rle``) with the strings written on the host."""
+    from . import engine
+    counts, begin = engine.bits_to_rle(bits, H, W, index)
+    return [{"size": [H, W], "counts": s} for s in counts_to_strings(counts, begin)]
+
+
+ENCODE_CHUNK = 256      # masks per host-to-device upload of encode_many (a 640x480 fp32 chunk is 315 MB)
+
+
+def encode_many(masks, device=None) -> list:
+    """``[encode(m) for m in masks]``, byte for byte, for an (n, H, W) fp32 / uint8 / bool stack of masks (numpy or
+    torch, host or CUDA).  Without a device (``device=None`` and host masks) that is what it does.  Otherwise
+    the masks are packed (``!= 0``, as ``encode`` tests them: NaN is set, -0.0 is not) and encoded on the GPU;
+    host masks are uploaded ``ENCODE_CHUNK`` at a time, so the dense stack never sits on the device whole."""
+    import torch
+    from . import engine
+    if isinstance(masks, np.ndarray):
+        masks = torch.from_numpy(masks)
+    if device is None and masks.is_cuda:
+        device = masks.device
+    n, H, W = masks.shape
+    if device is None or n == 0 or H * W == 0:
+        return [encode(m.numpy()) for m in masks.cpu()]
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise ValueError(f"encode_many encodes on a CUDA device, not {device}")
+    pool = engine.PoolBuilder(n, H, W, device, with_nonzero=True)
+    with torch.cuda.device(device):
+        for lo in range(0, n, ENCODE_CHUNK):
+            pool.append(masks[lo:lo + ENCODE_CHUNK].to(device))
+    return bits_to_rles(pool.nz, H, W)
+
+
 def rle_counts(rle: dict) -> np.ndarray:
     c = rle["counts"]
     if isinstance(c, (bytes, str)):

@@ -3,11 +3,14 @@ detections.  The R-CNN itself is out of scope (it stays in the reference's detec
 code); without it this tool runs on the synthetic detector stub (``synth.make_video``),
 which emits the same ``Instances`` contract:
 
-    python -m articulation3d_b200.tools.inference --frames 30 --tracks 4 --output out/ [--save-obj] [--save-textured-obj]
+    python -m articulation3d_b200.tools.inference --frames 30 --tracks 4 --output out/ [--save-obj] [--save-textured-obj] \
+        [--save-masks]
 
 ``--save-obj`` writes the geometry-only quads of ``io.write_obj``; ``--save-textured-obj`` the reference's export
 (``save_obj_model``, tools/inference.py:44-168, :282: object, rotated copies, axis markers, background, one
 300x300 texture each) through ``articulation3d_b200.export`` — with a flat grey image, the stub has no video.
+``--save-masks`` adds every fitted frame's registered mask to ``<id>_tracks.json`` as COCO RLE (``segmentation`` of
+each ``angle_track`` entry).
 """
 from __future__ import annotations
 
@@ -30,11 +33,12 @@ def main(argv=None):
     ap.add_argument("--device", default="cuda:0")
     ap.add_argument("--save-obj", action="store_true")
     ap.add_argument("--save-textured-obj", action="store_true")
+    ap.add_argument("--save-masks", action="store_true", help="registered masks (COCO RLE) in the tracks JSON")
     args = ap.parse_args(argv)
     random.seed(args.seed)                                   # tools/inference.py:172
     cfg = OptConfig()
     preds, _ = synth.make_video(args.seed, args.tracks, args.frames, cfg)
-    records = io.preds_to_records(preds, video_id="synthetic00_0_0")
+    records = io.preds_to_records(preds, video_id="synthetic00_0_0", device=args.device)
     torch.zeros(1, device=args.device)                       # CUDA context and library load are not the optimiser's time
     opt_utils._lib.load()
     torch.cuda.synchronize()
@@ -43,7 +47,8 @@ def main(argv=None):
     opt_preds = opt_utils.optimize_planes(preds, planes, '3dc', cfg=cfg, device=args.device)
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
-    io.save_results(args.output, "synthetic00_0_0", io.opt_preds_to_records(opt_preds, records), planes)
+    io.save_results(args.output, "synthetic00_0_0", io.opt_preds_to_records(opt_preds, records), planes,
+                    masks=args.save_masks)
     if args.save_obj:
         for k in sorted({0, min(30, args.frames - 1), min(60, args.frames - 1), min(89, args.frames - 1)}):
             io.write_obj(os.path.join(args.output, f"frame{k}.obj"), opt_preds, planes, k, cfg)   # inference.py:282

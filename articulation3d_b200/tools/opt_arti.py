@@ -1,13 +1,14 @@
 """Temporal optimisation of saved predictions — the B200 counterpart of the reference's
 ``tools/opt_arti.py`` for the stage in scope (the detector is not re-run):
 
-    python -m articulation3d_b200.tools.opt_arti --input instances_predictions.pth --output out/ [--save-obj]
+    python -m articulation3d_b200.tools.opt_arti --input instances_predictions.pth --output out/ [--save-obj] [--save-masks]
 
 Reads the per-frame prediction records (RLE masks stay run-length encoded and are decoded on
 the GPU), groups them by video, runs ``track_planes`` + ``optimize_planes('3dc')`` for all videos
 in lock-step, and writes per video ``<id>_predictions_opt.pth`` (records as
 tools/opt_arti.py:229-249), ``<id>_tracks.json`` (fitted axis + angle-per-frame track) and
-optionally ``<id>_frame<k>.obj``.  ``--synthetic N`` writes a synthetic input first.
+optionally ``<id>_frame<k>.obj``; ``--save-masks`` adds every fitted frame's registered mask to the tracks JSON
+as COCO RLE.  ``--synthetic N`` writes a synthetic input first (masks encoded on ``--device``).
 """
 from __future__ import annotations
 
@@ -34,6 +35,7 @@ def main(argv=None):
     ap.add_argument("--seed", type=int, default=2020, help="per-video RNG seed base (tools/inference.py:172)")
     ap.add_argument("--device", default="cuda:0")
     ap.add_argument("--save-obj", action="store_true")
+    ap.add_argument("--save-masks", action="store_true", help="registered masks (COCO RLE) in the tracks JSON")
     ap.add_argument("--gt-json", default=None, help="COCO-style ground truth: print the AP table before / after "
                     "optimisation (tools/opt_arti.py:275-283)")
     ap.add_argument("--synthetic", type=int, default=0, help="first write N synthetic videos to --input")
@@ -45,7 +47,8 @@ def main(argv=None):
         records = []
         for v in range(args.synthetic):
             preds, _ = synth.make_video(args.seed + v, args.tracks, args.frames)
-            records += io.preds_to_records(preds, video_id=f"synthetic{v:02d}_0_0", start_image_id=v * 10000)
+            records += io.preds_to_records(preds, video_id=f"synthetic{v:02d}_0_0", start_image_id=v * 10000,
+                                           device=args.device)
         torch.save(records, args.input)
 
     cfg = OptConfig()
@@ -62,7 +65,7 @@ def main(argv=None):
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     for (vid, recs), (preds, planes), out in zip(order, videos, outs):
-        io.save_results(args.output, vid, io.opt_preds_to_records(out, recs), planes)
+        io.save_results(args.output, vid, io.opt_preds_to_records(out, recs), planes, masks=args.save_masks)
         if args.save_obj:
             for k in (0, len(preds) // 3, 2 * len(preds) // 3, len(preds) - 1):
                 io.write_obj(os.path.join(args.output, f"{vid}_frame{k}.obj"), out, planes, k, cfg)

@@ -257,6 +257,28 @@ int a3d_emit_masks(const uint32_t* bits, const int32_t* index, int64_t n, int H,
 int a3d_rle_to_bits(const uint32_t* counts, const int64_t* begin, int64_t n, int H, int W,
                     uint32_t* bits, void* stream);
 
+/* (f2, SURVEY.md 8f) packed masks -> COCO RLE run lengths on the device, the inverse of a3d_rle_to_bits: the
+ * `counts` rle.encode computes (pycocotools mask_util.encode in the reference), runs alternating 0/1 in
+ * column-major order, starting with 0s (a set pixel (0,0) gives a first run of 0); every mask's runs sum to
+ * H*W.  Two calls, both asynchronous on `stream`; `index` selects the masks as in a3d_emit_masks (NULL =
+ * identity).  Any H, W >= 1 with H*W <= 2^31 - 1 (A3D_ELIMIT beyond), any n.
+ *   runs_out   [n] int64: number of runs of every selected mask (first call)
+ *   begin      [n+1] int64: exclusive scan of runs_out (begin[0] = 0)
+ *   counts_out [begin[n]] uint32: mask i's runs go to counts_out[begin[i] .. begin[i+1])               */
+int a3d_rle_count_runs(const uint32_t* bits, const int32_t* index, int64_t n, int H, int W,
+                       int64_t* runs_out, void* stream);
+int a3d_bits_to_rle(const uint32_t* bits, const int32_t* index, int64_t n, int H, int W,
+                    const int64_t* begin, uint32_t* counts_out, void* stream);
+
+/* HOST helper: COCO compressed strings of n masks' run lengths (the inverse of a3d_host_rle_counts; byte for
+ * byte what rle.counts_to_string writes).
+ *   counts          HOST uint32, mask i's runs at counts[begin[i] .. begin[i+1]);  begin  HOST [n+1]
+ *   chars_out       HOST [cap] (7 * total counts always suffices)
+ *   char_begin_out  HOST [n+1] first byte of every mask's string (may be NULL)
+ * Returns the total number of bytes, or a negative A3D_E* code (bad offsets, cap too small).          */
+int64_t a3d_host_rle_strings(const uint32_t* counts, const int64_t* begin, int64_t n,
+                             uint8_t* chars_out, int64_t cap, int64_t* char_begin_out);
+
 /* (f1, SURVEY.md 8f) plane offset implied by the depth map: for every instance the mean
  * over its mask of normal . (rays * depth).  Replaces the per-instance loop of
  * override_depth (utils/arti_vis.py:125-149) and depth2XYZ (:90-99).
