@@ -13,6 +13,8 @@
 """
 from __future__ import annotations
 
+import zipfile
+
 import numpy as np
 import torch
 
@@ -135,9 +137,11 @@ def override_depth_batch(instances, depths: torch.Tensor | None = None, xyzs=Non
     return instances
 
 
-def load_predictions(path: str):
-    """``instances_predictions.pth``: list of per-keyframe dicts (tools/opt_arti.py:56-57)."""
-    return torch.load(path, map_location="cpu", weights_only=False)
+def load_predictions(path: str, mmap: bool = False):
+    """``instances_predictions.pth``: list of per-keyframe dicts (tools/opt_arti.py:56-57).  ``mmap=True`` maps the
+    tensors' storages from the file instead of reading them, so processes loading the same file share its pages;
+    a file in torch's legacy (non-zip) format cannot be mapped and is read."""
+    return torch.load(path, map_location="cpu", weights_only=False, mmap=mmap and zipfile.is_zipfile(path))
 
 
 def video_key(file_name: str):
