@@ -7,12 +7,14 @@
 * ``override_depth`` — replaces every instance's plane offset by the mean over its
   mask of ``normal . XYZ`` (reference utils/arti_vis.py:125-149, with ``depth2XYZ``
   :90-99 and ``get_K_inv_dot_xy_1`` :101-122), as one device launch for all
-  instances of all frames handed in.
+  instances of all frames handed in; ``override_depth_records`` does the same for records carrying
+  ``pred_depth``, streaming the depth through the device in bounded chunks.
 * ``load_predictions`` / ``group_by_video`` — the ``instances_predictions.pth``
   record list of tools/opt_arti.py:56-76.
 """
 from __future__ import annotations
 
+import functools
 import zipfile
 
 import numpy as np
@@ -135,6 +137,129 @@ def override_depth_batch(instances, depths: torch.Tensor | None = None, xyzs=Non
             inst["pred_plane"] = new[k:k + n].clone()
         k += n
     return instances
+
+
+@functools.lru_cache(maxsize=None)
+def _depth_rays(H: int, W: int, device: torch.device) -> torch.Tensor:
+    return torch.FloatTensor(get_K_inv_dot_xy_1(H, W)).to(device)
+
+
+def check_depth_records(records):
+    """Raise ``ValueError`` naming the record's ``file_name`` if a record carries no ``pred_depth``, if its
+    ``pred_plane`` rows differ from its number of instances, or if its depth map is not the (H, W) of its masks'
+    ``segmentation.size``.  Host-side only: no library load, no device use."""
+    for r in records:
+        name = r.get("file_name")
+        if "pred_depth" not in r:
+            raise ValueError(f"{name}: the record carries no pred_depth to override its planes from")
+        n = len(r["instances"])
+        if r["pred_plane"].dim() != 2 or r["pred_plane"].shape[0] != n:
+            raise ValueError(f"{name}: pred_plane has shape {list(r['pred_plane'].shape)} for {n} instance(s)")
+        sizes = {tuple(int(x) for x in d["segmentation"]["size"]) for d in r["instances"]}
+        if len(sizes) > 1:
+            raise ValueError(f"{name}: the masks mix frame sizes {sorted(sizes)}")
+        if sizes and tuple(r["pred_depth"].shape) != next(iter(sizes)):
+            raise ValueError(f"{name}: pred_depth has shape {list(r['pred_depth'].shape)}, "
+                             f"the masks are {list(next(iter(sizes)))}")
+
+
+def override_depth_records(records, device, chunk_bytes: int = 256 << 20):
+    """``override_depth_batch`` of ``records`` (reference-format records carrying ``pred_depth``, possibly
+    memory-mapped) with the depth streamed through the device in chunks, so device memory stays bounded by two
+    chunks of depth plus one chunk's mask pool whatever the number of records.  Replaces every record's
+    ``pred_plane`` in place, with the same quirks as ``override_depth_batch`` (the input plane tensor is swapped in
+    place, an empty mask keeps its plane, records without instances pass through) and bit for bit the same values:
+    ``k_plane_offsets`` reduces each instance in one CTA in a fixed order, so the chunking changes no value.
+
+    Consecutive frames with instances form a chunk while their fp32 depth fits ``chunk_bytes`` (at least one
+    frame) and their size does not change.  A chunk's depth maps are copied into one of two pinned staging
+    blocks and sent on a side stream, so the copy of chunk k+1 runs while chunk k is decoded (one
+    ``rle_to_pool``) and reduced (one ``plane_offsets``).  Offsets and counts stay on the device until one
+    D2H copy at the end.  Every record is checked (``check_depth_records``) before any device work."""
+    check_depth_records(records)
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise engine._lib.A3DError("override_depth needs a CUDA device (no CPU fallback)")
+    planes = []
+    for r in records:
+        p = r["pred_plane"]
+        p[:, [1, 2]] = p[:, [2, 1]]                     # in place, as the reference (:129-130)
+        p[:, 1] = -p[:, 1]
+        planes.append(p)
+    frames = [r for r in records if r["instances"]]
+    if not frames:
+        return records
+    planes_t = torch.cat(planes).float()
+    offset = torch.linalg.vector_norm(planes_t, dim=1)
+    normal = planes_t / offset.clamp_min(1e-8)[:, None]
+
+    chunks, first = [], 0                               # (first frame, frames, first instance, instances, H, W)
+    n_inst = 0
+    for i, r in enumerate(frames):
+        H, W = r["pred_depth"].shape
+        if i > first and ((H, W) != tuple(chunks[-1][4:]) or (i - first + 1) * H * W * 4 > chunk_bytes):
+            first = i
+        if i == first:
+            chunks.append([i, 0, n_inst, 0, H, W])
+        chunks[-1][1] += 1
+        chunks[-1][3] += len(r["instances"])
+        n_inst += len(r["instances"])
+    stage_elems = max(c[1] * c[4] * c[5] for c in chunks)
+
+    with torch.cuda.device(device):
+        main, side = torch.cuda.current_stream(), torch.cuda.Stream()
+        normal_d = normal.to(device)
+        pinned = [torch.empty(stage_elems, dtype=torch.float32, pin_memory=True) for _ in range(min(2, len(chunks)))]
+        depth_d = [torch.empty(stage_elems, dtype=torch.float32, device=device) for _ in pinned]
+        copied = [torch.cuda.Event() for _ in pinned]      # H2D of the slot's block done
+        consumed = [None] * len(pinned)                     # launches reading the slot's device block enqueued
+
+        def stage(k):
+            s = k % len(pinned)
+            f0, nf, _, _, H, W = chunks[k]
+            copied[s].synchronize()                         # the block's previous H2D has read it
+            host = pinned[s][:nf * H * W].view(nf, H, W)
+            for j in range(nf):
+                host[j].copy_(torch.as_tensor(frames[f0 + j]["pred_depth"]))
+            with torch.cuda.stream(side):
+                if consumed[s] is not None:
+                    side.wait_event(consumed[s])
+                depth_d[s][:nf * H * W].copy_(pinned[s][:nf * H * W], non_blocking=True)
+                copied[s].record(side)
+
+        parts_off, parts_cnt = [], []
+        stage(0)
+        for k, (f0, nf, i0, ni, H, W) in enumerate(chunks):
+            if k + 1 < len(chunks):
+                stage(k + 1)
+            s = k % len(pinned)
+            rles, frame_of = [], []
+            for j in range(nf):
+                for det in frames[f0 + j]["instances"]:
+                    rles.append(det["segmentation"])
+                    frame_of.append(j)
+            pool = engine.rle_to_pool(rles, H, W, device)
+            main.wait_event(copied[s])
+            off, cnt = engine.plane_offsets(pool, torch.arange(ni, dtype=torch.int32, device=device),
+                                            normal_d[i0:i0 + ni], _depth_rays(H, W, device),
+                                            depth_d[s][:nf * H * W].view(nf, H, W),
+                                            torch.tensor(frame_of, dtype=torch.int32, device=device))
+            consumed[s] = torch.cuda.Event()
+            consumed[s].record(main)
+            parts_off.append(off)
+            parts_cnt.append(cnt)
+            del pool
+        res = torch.cat([torch.cat(parts_off).view(torch.int32), torch.cat(parts_cnt)]).cpu()
+    off, cnt = res[:n_inst].view(torch.float32), res[n_inst:]
+    new = torch.where((cnt > 0)[:, None], normal * off[:, None], planes_t)       # empty mask keeps the plane
+    new[:, [1, 2]] = new[:, [2, 1]]
+    new[:, 2] = -new[:, 2]
+    k = 0
+    for r in frames:
+        n = len(r["instances"])
+        r["pred_plane"] = new[k:k + n].clone()
+        k += n
+    return records
 
 
 def load_predictions(path: str, mmap: bool = False):

@@ -20,9 +20,10 @@ from . import adapter, geometry, rle
 from .config import OptConfig
 
 
-def preds_to_records(preds, video_id: str = "synthetic00_0_0", start_image_id: int = 0, device=None):
+def preds_to_records(preds, video_id: str = "synthetic00_0_0", start_image_id: int = 0, device=None, depths=None):
     """list[Instances] (dense masks) -> list of reference-format records (RLE masks).  With a CUDA ``device`` the
-    masks are thresholded (``> 0.5``), packed and encoded there, with the same records as a result."""
+    masks are thresholded (``> 0.5``), packed and encoded there, with the same records as a result.  ``depths``
+    ((T,H,W), e.g. ``synth.render_depths``) is stored per frame as ``pred_depth`` (fp32, on the host)."""
     segs = None
     if device is not None:
         segs = iter(_encode_preds_on_device(preds, torch.device(device)))
@@ -39,6 +40,8 @@ def preds_to_records(preds, video_id: str = "synthetic00_0_0", start_image_id: i
         records.append({"image_id": start_image_id + t, "file_name": f"{video_id}_{t}.png", "instances": inst,
                         "pred_plane": p.pred_planes.clone(), "pred_rot_axis": p.pred_rot_axis.clone(),
                         "pred_tran_axis": p.pred_tran_axis.clone()})
+        if depths is not None:
+            records[-1]["pred_depth"] = depths[t].to("cpu", torch.float32).clone()
     return records
 
 

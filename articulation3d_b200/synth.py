@@ -244,6 +244,41 @@ def make_video(seed: int, n_tracks: int, n_frames: int, cfg: OptConfig | None = 
     return preds, scene
 
 
+def scene_planes(scene: VideoScene) -> torch.Tensor:
+    """(N,T,3) float64 true plane vectors ``n * offset`` of every track and frame, camera axes (x right, y down,
+    z forward), without the detector's ``plane_jitter``."""
+    n = torch.cross(scene.d[:, None, :].expand_as(scene.w), scene.w, dim=2)
+    return n * (n * scene.hinge).sum(2, keepdim=True)
+
+
+def scene_pred_planes(scene: VideoScene) -> torch.Tensor:
+    """``scene_planes`` in the records' ``pred_plane`` axes (as ``track_predictions`` writes them), fp32."""
+    c = scene_planes(scene)
+    return torch.stack([c[..., 0], c[..., 2], -c[..., 1]], -1).to(torch.float32)
+
+
+def render_depths(scene: VideoScene, cfg: OptConfig | None = None, device="cpu",
+                  background: float = 10.0) -> torch.Tensor:
+    """(T,H,W) fp32 depth maps of a clip, as the records' ``pred_depth``: every pixel's ray of the depth camera
+    (``adapter.get_K_inv_dot_xy_1(H, W)``, z = 1) meets the true plane (``scene_planes``) of each track whose mask
+    (``render_track_masks``) covers the pixel; the nearest intersection in front of the camera wins, and a pixel
+    no track covers that way gets ``background``."""
+    from .adapter import get_K_inv_dot_xy_1
+    cfg = cfg or OptConfig()
+    H, W = cfg.height, cfg.width
+    rays = torch.from_numpy(get_K_inv_dot_xy_1(H, W)).to(device)                   # (3,H,W) float64
+    planes = scene_planes(scene).to(device)                                         # (N,T,3)
+    depth = torch.full((scene.n_frames, H, W), math.inf, dtype=torch.float64, device=device)
+    for k in range(planes.shape[0]):
+        masks = render_track_masks(scene, k, cfg, device=device)
+        off = planes[k].norm(dim=1)                                                 # plane: normal . X = off
+        normal = planes[k] / off[:, None]
+        t = off[:, None, None] / torch.einsum("tc,chw->thw", normal, rays)
+        hit = masks & (t > 0) & torch.isfinite(t)
+        depth = torch.where(hit, torch.minimum(depth, t), depth)
+    return torch.where(torch.isinf(depth), background, depth).to(torch.float32)
+
+
 def clone_preds(preds, instances_cls=Instances, boxes_cls=Boxes):
     """Deep copy of a prediction list, optionally re-typed (e.g. into the shim
     classes the unmodified reference is run with)."""

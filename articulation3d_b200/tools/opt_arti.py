@@ -9,8 +9,10 @@ the GPU), groups them by video, runs ``track_planes`` + ``optimize_planes('3dc')
 in lock-step, and writes per video ``<id>_predictions_opt.pth`` (records as
 tools/opt_arti.py:229-249), ``<id>_tracks.json`` (fitted axis + angle-per-frame track) and
 optionally ``<id>_frame<k>.obj``; ``--save-masks`` adds every fitted frame's registered mask to the tracks JSON
-as COCO RLE.  ``--synthetic N`` writes a synthetic input first (masks encoded on the tool's GPU; under torchrun
-rank 0 writes it on its own).  The camera is the reference's 640x480 one scaled to the records' frame size
+as COCO RLE.  ``--override-depth`` first replaces every instance's plane offset by the one its record's
+``pred_depth`` implies (the reference's ``override_depth``), streamed through the GPU per rank.  ``--synthetic N``
+writes a synthetic input first (masks encoded on the tool's GPU; under torchrun rank 0 writes it on its own;
+``--synthetic-depth`` adds a rendered ``pred_depth``).  The camera is the reference's 640x480 one scaled to the records' frame size
 (``segmentation.size``).
 
 Under torchrun (WORLD_SIZE > 1) rank r runs on cuda:$LOCAL_RANK and converts, tracks, optimises and writes
@@ -72,9 +74,16 @@ def main(argv=None):
                     "optimisation (tools/opt_arti.py:275-283)")
     ap.add_argument("--synthetic", type=int, default=0, help="first write N synthetic videos to --input "
                     "(masks encoded on the tool's GPU; under torchrun rank 0 writes)")
+    ap.add_argument("--synthetic-depth", action="store_true", help="with --synthetic: the records carry a "
+                    "rendered pred_depth (synth.render_depths)")
+    ap.add_argument("--override-depth", action="store_true", help="replace every instance's plane offset by the "
+                    "mean over its mask of normal . XYZ of the record's pred_depth before tracking "
+                    "(adapter.override_depth_records; tools/inference.py:220, tools/opt_arti.py:173-185)")
     ap.add_argument("--tracks", type=int, default=4)
     ap.add_argument("--frames", type=int, default=60)
     args = ap.parse_args(argv)
+    if args.synthetic_depth and not args.synthetic:
+        ap.error("--synthetic-depth needs --synthetic N")
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world == 1:
@@ -91,13 +100,53 @@ def main(argv=None):
         dist.destroy_process_group()
 
 
+def _override_depth(args, order, mine, rank: int, world: int, device: torch.device):
+    """``adapter.override_depth_records`` of this rank's block of videos, in place.  Every rank checks every record
+    first, so a bad record anywhere stops all ranks before any device work.  With ``--gt-json`` under torchrun,
+    rank 0 receives the other blocks' new planes (one gather) for its "before" table.  Rank 0 prints frames,
+    instances and depth bytes over all ranks, and the slowest rank's override time."""
+    adapter.check_depth_records([r for _, recs in order for r in recs])
+    block = [r for i in mine for r in order[i][1]]
+    t0 = time.perf_counter()
+    adapter.override_depth_records(block, device)           # ends in a D2H copy of the results
+    dt = time.perf_counter() - t0
+    counts = [len(block), sum(len(r["instances"]) for r in block),
+              sum(r["pred_depth"].numel() * 4 for r in block if r["instances"])]
+    where = ""
+    if world > 1:
+        total = torch.tensor(counts, dtype=torch.int64, device=device)
+        dist.all_reduce(total)
+        slowest = torch.tensor([dt], dtype=torch.float64, device=device)
+        dist.all_reduce(slowest, op=dist.ReduceOp.MAX)
+        counts, dt, where = total.tolist(), slowest.item(), f" on {world} GPUs"
+        if args.gt_json:
+            local = torch.cat([torch.zeros(0, 3)] + [r["pred_plane"].to(torch.float32) for r in block])
+            local = local.view(torch.int32)
+            if dist.get_backend() == "nccl":
+                local = local.to(device)
+            rows = a3d_dist.all_gather_rows(local).cpu().view(torch.float32)
+            if rank == 0:
+                k = 0
+                for _, recs in order:
+                    for r in recs:
+                        n = len(r["instances"])
+                        if n:
+                            r["pred_plane"] = rows[k:k + n].clone()
+                        k += n
+    if rank == 0:
+        frames, instances, nbytes = counts
+        print(f"override-depth: {frames} frame(s), {instances} instance(s), {nbytes / 1e6:.1f} MB of depth "
+              f"in {dt * 1e3:.1f} ms{where}")
+
+
 def _run(args, rank: int, world: int, device: torch.device):
     if args.synthetic and rank == 0:
         records = []
         for v in range(args.synthetic):
-            preds, _ = synth.make_video(args.seed + v, args.tracks, args.frames)
+            preds, scene = synth.make_video(args.seed + v, args.tracks, args.frames)
+            depths = synth.render_depths(scene) if args.synthetic_depth else None
             records += io.preds_to_records(preds, video_id=f"synthetic{v:02d}_0_0", start_image_id=v * 10000,
-                                           device=device)
+                                           device=device, depths=depths)
         torch.save(records, args.input)
     if world > 1:
         dist.barrier()
@@ -106,6 +155,8 @@ def _run(args, rank: int, world: int, device: torch.device):
     order = list(adapter.group_by_video(adapter.load_predictions(args.input, mmap=world > 1)).items())
     cfg = frame_config(dict(order))
     mine = a3d_dist.shard_range(len(order), rank, world)
+    if args.override_depth:
+        _override_depth(args, order, mine, rank, world, device)
     videos = [None] * len(order)                  # only this rank's block is converted and tracked
     for i in mine:
         preds = io.records_to_preds(order[i][1], conf_threshold=args.conf_threshold, masks="rle")
