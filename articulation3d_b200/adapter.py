@@ -86,9 +86,22 @@ def override_depth(instance: dict, depth: torch.Tensor | None = None, xyz: torch
 
 def override_depth_batch(instances, depths: torch.Tensor | None = None, xyzs=None,
                          rays: torch.Tensor | None = None, device=None):
-    """All frames at once: one RLE decode launch + one masked-mean launch."""
+    """All frames at once: one RLE decode launch + one masked-mean launch.  ``depths`` is (len(instances), H, W),
+    ``xyzs`` one (3, H, W) map per frame and ``rays`` (3, H, W), with (H, W) the masks' size; other shapes are
+    refused before any device use (the maps are indexed by frame position)."""
     if (depths is None) == (xyzs is None):
         raise ValueError("give exactly one of depths / xyzs")
+    sizes = [det["segmentation"]["size"] for inst in instances for det in inst["instances"]]
+    if sizes:
+        H, W = (int(s) for s in sizes[0])
+        maps = [("depths", depths, [len(instances), H, W]), ("rays", rays, [3, H, W])]
+        if xyzs is not None:
+            if len(xyzs) != len(instances):
+                raise ValueError(f"{len(xyzs)} xyzs map(s) for {len(instances)} frame(s)")
+            maps += [(f"xyzs[{f}]", x, [3, H, W]) for f, x in enumerate(xyzs)]
+        for name, t, shape in maps:
+            if t is not None and list(t.shape) != shape:
+                raise ValueError(f"{name} has shape {list(t.shape)}, the masks need {shape}")
     if device is None:
         device = (depths if depths is not None else xyzs[0]).device
     device = torch.device(device)
@@ -105,7 +118,6 @@ def override_depth_batch(instances, depths: torch.Tensor | None = None, xyzs=Non
             planes.append(p[k])
     if not rles:
         return instances
-    H, W = rles[0]["size"]
     pool = engine.rle_to_pool(rles, H, W, device)
     planes_t = torch.stack(planes).float()
     offset = torch.linalg.vector_norm(planes_t, dim=1)
@@ -114,7 +126,7 @@ def override_depth_batch(instances, depths: torch.Tensor | None = None, xyzs=Non
     if depths is not None:
         if rays is None:
             rays = torch.FloatTensor(get_K_inv_dot_xy_1(H, W)).to(device)
-        off, cnt = engine.plane_offsets(pool, idx, normal.to(device), rays.to(device), depths.to(device).reshape(-1, H, W),
+        off, cnt = engine.plane_offsets(pool, idx, normal.to(device), rays.to(device), depths.to(device),
                                         torch.tensor(frame_of, dtype=torch.int32, device=device))
     else:
         # one launch per distinct XYZ map (the reference signature hands in one frame at a time)
@@ -124,7 +136,7 @@ def override_depth_batch(instances, depths: torch.Tensor | None = None, xyzs=Non
         for f, xyz in enumerate(xyzs):
             sel = (fo == f).nonzero()[:, 0]
             if sel.numel():
-                o, c = engine.plane_offsets(pool, idx[sel], normal[sel.cpu()].to(device), xyz.to(device).reshape(3, H, W))
+                o, c = engine.plane_offsets(pool, idx[sel], normal[sel.cpu()].to(device), xyz.to(device))
                 off[sel], cnt[sel] = o, c
     off, cnt = off.cpu(), cnt.cpu()
     new = torch.where((cnt > 0)[:, None], normal * off[:, None], planes_t)       # empty mask keeps the plane

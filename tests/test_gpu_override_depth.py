@@ -86,6 +86,56 @@ def test_records_match_reference_at_768x1024():
         np.testing.assert_allclose(r["pred_plane"].numpy(), ref.numpy(), rtol=1e-4, atol=1e-6)
 
 
+MIXED = [(480, 640)] * 3 + [(29, 1057)] * 2 + [None] + [(480, 640)] * 2 + [(768, 1024)]
+
+
+def _mixed_records(seed=3):
+    """Records of changing frame sizes (``MIXED``; None: a 480x640 record without instances) with edge and blob
+    masks, random planes and random fp32 depth; plus each record's masks."""
+    from tests.test_gpu_plane_offsets import edge_masks
+    rng = np.random.RandomState(seed)
+    records, masks = [], []
+    for t, size in enumerate(MIXED):
+        H, W = size or (480, 640)
+        e = edge_masks(H, W, rng)
+        m = e[rng.permutation(len(e))[:4 + t % 3]] if size else e[:0]
+        records.append({"file_name": f"mixed_{t}.png", "instances": [{"segmentation": rle.encode(x)} for x in m],
+                        "pred_plane": torch.from_numpy(rng.normal(size=(len(m), 3)).astype(np.float32)),
+                        "pred_depth": torch.from_numpy(rng.uniform(0.5, 4, (H, W)).astype(np.float32))})
+        masks.append(m)
+    return records, masks
+
+
+@pytest.mark.parametrize("chunk_bytes", [1, 2 * 768 * 1024 * 4, 1 << 40], ids=["1_frame", "2_largest", "all"])
+def test_records_of_mixed_sizes(chunk_bytes):
+    """Chunks end where the frame size changes: the planes are bit-equal to ``override_depth_batch`` of each
+    same-size group and within the bound of the float64 reference (tests/test_gpu_plane_offsets.py), whatever
+    the chunk size."""
+    from tests.test_gpu_plane_offsets import assert_planes, reference_planes
+    records, masks = _mixed_records()
+    inputs = [r["pred_plane"].clone() for r in records]
+    groups = {}
+    for i, r in enumerate(records):
+        if r["instances"]:
+            groups.setdefault(tuple(r["pred_depth"].shape), []).append(i)
+    want = {}
+    for (H, W), idx in groups.items():
+        recs = [dict(records[i], pred_plane=inputs[i].clone()) for i in idx]
+        out = adapter.override_depth_batch(recs, depths=torch.stack([r["pred_depth"] for r in recs]).to(DEV))
+        want.update({i: r["pred_plane"] for i, r in zip(idx, out)})
+        rays = adapter.get_K_inv_dot_xy_1(H, W).astype(np.float32)
+        frame_of = np.concatenate([np.full(len(masks[i]), k) for k, i in enumerate(idx)])
+        ref = reference_planes(torch.cat([inputs[i] for i in idx]), np.concatenate([masks[i] for i in idx]),
+                               frame_of, rays, np.stack([records[i]["pred_depth"].numpy() for i in idx]))
+        assert_planes(torch.cat([want[i] for i in idx]), ref, f"{H}x{W}")
+    adapter.override_depth_records(records, DEV, chunk_bytes=chunk_bytes)
+    for i, r in enumerate(records):
+        if i in want:
+            assert torch.equal(r["pred_plane"].view(torch.int32), want[i].view(torch.int32)), r["file_name"]
+        else:
+            assert r["pred_plane"].shape == (0, 3)
+
+
 def test_memory_mapped_file_is_unchanged(tmp_path):
     path = str(tmp_path / "pred.pth")
     torch.save(_records(480, 640), path)

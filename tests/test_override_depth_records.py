@@ -70,6 +70,39 @@ def test_tool_refuses_before_device_work(kind, words, tmp_path, monkeypatch):
     assert not os.path.exists(out)
 
 
+MAPS = [("fewer_depths", ["[2, 48, 64]", "[3, 48, 64]"]), ("transposed_depths", ["[3, 64, 48]", "[3, 48, 64]"]),
+        ("flat_depths", ["[3, 3072]", "[3, 48, 64]"]), ("xyz_shape", ["xyzs[1]", "[3, 64, 48]", "[3, 48, 64]"]),
+        ("fewer_xyzs", ["2 xyzs", "3 frame"]), ("rays_shape", ["rays", "[3, 64, 48]", "[3, 48, 64]"])]
+
+
+@pytest.mark.parametrize("kind,words", MAPS, ids=[k for k, _ in MAPS])
+def test_batch_refuses_maps_that_do_not_match_before_device_work(kind, words, monkeypatch):
+    """``override_depth_batch`` indexes the maps by frame position: a stack of the wrong size or orientation is
+    refused, naming both shapes, before the device check and any library use, with no plane swapped."""
+    recs = _records()
+    depths, xyzs, rays = torch.ones(3, 48, 64), None, None
+    if kind == "fewer_depths":
+        depths = depths[:2]
+    elif kind == "transposed_depths":
+        depths = depths.transpose(1, 2)
+    elif kind == "flat_depths":
+        depths = depths.reshape(3, -1)
+    elif kind == "rays_shape":
+        rays = torch.ones(3, 64, 48)
+    else:
+        depths, xyzs = None, [torch.ones(3, 48, 64) for _ in recs]
+        if kind == "xyz_shape":
+            xyzs[1] = torch.ones(3, 64, 48)
+        else:
+            xyzs = xyzs[:2]
+    _no_device(monkeypatch)
+    planes = [r["pred_plane"].clone() for r in recs]
+    with pytest.raises(ValueError) as e:
+        adapter.override_depth_batch(recs, depths=depths, xyzs=xyzs, rays=rays, device="cuda:0")
+    assert all(w in str(e.value) for w in words), str(e.value)
+    assert all(torch.equal(r["pred_plane"], p) for r, p in zip(recs, planes))
+
+
 def test_records_without_instances_need_no_size_match():
     recs = _records(n=0)
     recs[0]["pred_depth"] = torch.ones(3, 5)

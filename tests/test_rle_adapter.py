@@ -70,9 +70,13 @@ def test_create_instances_contract():
 
 
 def test_ray_table_matches_reference_loop_on_a_subgrid():
-    a = adapter.get_K_inv_dot_xy_1(48, 64)
-    b = restated.get_K_inv_dot_xy_1(48, 64)
-    assert np.array_equal(a, b)
+    """The vectorised table is the reference's double loop bit for bit at every frame size the tool and the depth
+    override use it at: odd and 1-pixel sizes, rows wider than 1024."""
+    for h, w in ((48, 64), (37, 1057), (1, 1), (768, 1024)):
+        a = adapter.get_K_inv_dot_xy_1(h, w)
+        b = restated.get_K_inv_dot_xy_1(h, w)
+        assert a.shape == (3, h, w)
+        assert np.array_equal(a, b), (h, w)
 
 
 def test_native_string_decoder_equals_python_decoder():
