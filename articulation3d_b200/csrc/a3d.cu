@@ -1606,48 +1606,57 @@ k_score_tma(const __grid_constant__ TmaMaps maps, const a3d_job_t* __restrict__ 
 // score on the tensor cores.  inter[t][c] = sum over pixels of T_t[p] * P_c[p] is a dense
 // contraction with 1-bit operands: a (targets x pixels) . (pixels x candidates) product.  Blackwell
 // has no 1-bit MMA (mma.sync .b1 is emulated with IMMA on sm_100a), so the words of the overlap
-// region are expanded to 0/1 bytes in shared memory and fed to tcgen05.mma kind::i8
-// (u8 x u8 -> s32, exact), accumulating a 128 x N tile in tensor memory.
+// region are expanded to 4-bit e2m1 values (bit -> 0x2 = 1.0) in shared memory and fed to
+// tcgen05.mma kind::mxf4 with every UE8M0 block scale 1.0: each product is exactly 0 or 1 and the
+// f32 accumulator of the 128 x N tile in tensor memory holds every count below 2^24 exactly
+// (tools/mma_probe.cu checks this past 2^21; a3d_score takes k_score for frames over 2^24 pixels).
 //   * CTA = (job, 128 targets, N <= 240 candidates); region = (hull of its target boxes) ∩ (hull of
-//     its candidate boxes), walked as one row-major sequence of word positions, 4 per step.
-//   * 24 producer warps: thread -> (word of the step, up to 2 masks).  One 4-byte load per word, issued
-//     8 steps ahead of its use (register ring, static indices through unrolling); 8 shift+mask ops turn the
-//     word into 32 bytes (byte 4j+i of the K=32 slice = bit j+8i — any permutation serves as long as both
-//     operands use it); two 16-byte stores into the no-swizzle K-major core-matrix layout
-//     [K chunk of 16 B][row][16 B] (LBO = rows*16, SBO = 128; tools/mma_probe.cu pins the fields);
-//     fence.proxy.async; arrive on the stage's full barrier.
-//   * one thread issues one MMA (K = 32 bytes = one word position) per position of the step and commits
-//     the stage back to the producers (4 stages).
+//     its candidate boxes), walked as one row-major sequence of word positions, 16 per step.
+//   * 24 producer warps: thread -> (word of the step, up to 8 masks).  One 4-byte load per word, issued
+//     2 steps ahead of its use (register ring, static indices through unrolling); 4 shift+mask ops turn
+//     the word into 16 bytes of nibbles (nibble i of register j = bit 4i+j — any permutation serves as
+//     long as both operands use it); one 16-byte store into the no-swizzle K-major core-matrix layout
+//     [word position][row][16 B]; fence.proxy.async; arrive on the stage's full barrier.
+//   * one thread issues one MMA (K = 64 = two word positions: LBO = the position slot, SBO = 128;
+//     tools/mma_probe.cu pins the fields) per position pair of the step and commits the stage back to
+//     the producers (2 stages of 16 positions).  An odd last position is paired with zeros.
+//   * block scales: 0x7F (2^0) in every byte of TMEM columns 256..511, written once per CTA.
 //   * epilogue: warps 0-3 read their 32 TMEM lanes (= targets) with tcgen05.ld, and every thread
 //     scans its target's candidates: union, fp32 divide, arg-max key, one atomicMax per target.
-// Bound (DESIGN.md §4): shared-memory bandwidth — every mask bit crosses shared memory as a byte twice
-// (producer store, tensor-core operand read: 2 x 10 KB per word position at N = 192).  A variant with
-// dedicated loader warps and a raw-word ring measured slower (650 vs 440 us on the C3 shard), an L2
-// prefetch of the rows ahead made no difference: the loads are not the limit.
+// Bound (DESIGN.md §4): shared-memory bandwidth — every mask bit crosses shared memory as a nibble
+// twice (producer store, tensor-core operand read: 2 x 5 KB per word position at N = 192).
 // ---------------------------------------------------------------------------
 #ifndef A3D_MMA_WARPS
 #define A3D_MMA_WARPS 24
 #endif
 #ifndef A3D_MMA_AHEAD
-#define A3D_MMA_AHEAD 8
+#define A3D_MMA_AHEAD 2
+#endif
+#ifndef A3D_MMA_POS
+#define A3D_MMA_POS 16
+#endif
+#ifndef A3D_MMA_STAGES
+#define A3D_MMA_STAGES 2
 #endif
 constexpr int kMmaProducerWarps = A3D_MMA_WARPS;
 constexpr int kMmaProducers = 32 * kMmaProducerWarps;
 constexpr int kMmaThreads = kMmaProducers + 32;   // + the issuing warp
 constexpr int kMmaM = 128;                    // targets per CTA (TMEM lanes)
 constexpr int kMmaNMax = 240;                 // candidates per CTA (TMEM columns), multiple of 16
-constexpr int kMmaStages = 4;
-constexpr int kMmaPos = 4;                    // word positions per stage
+constexpr int kMmaStages = A3D_MMA_STAGES;
+constexpr int kMmaPos = A3D_MMA_POS;          // word positions per stage (two per MMA)
 constexpr int kMmaItems = ((kMmaM + kMmaNMax) * kMmaPos + kMmaProducers - 1) / kMmaProducers;   // words per producer thread per step
-constexpr int kMmaABlock = 2 * kMmaM * 16;    // bytes of one position of A
-constexpr int kMmaTmemCols = 256;
+constexpr int kMmaTmemCols = 512;             // accumulator in columns 0..255, block scales in 256..511
+constexpr int kMmaSfCol = 256;
 constexpr int kMmaAhead = A3D_MMA_AHEAD;                  // steps between a producer's loads and its stores
+static_assert(kMmaPos >= 2 && (kMmaPos & (kMmaPos - 1)) == 0 && kMmaProducers % kMmaPos == 0,
+              "positions of a step pair up into MMAs; a thread's word is tid & (kMmaPos - 1)");
 
-// position blocks of one stage are padded by 32 bytes so that the 16-byte stores of a quarter-warp
-// (4 words of one mask, then of the next mask) hit distinct banks
-constexpr int kMmaPad = 32;
+// position slots of one stage are padded so that the 16-byte stores of a quarter-warp (8 positions
+// of one mask, or 4 positions of two masks) hit distinct banks
+constexpr int kMmaPad = kMmaPos >= 8 ? 16 : 32;
 __host__ __device__ constexpr size_t mma_stage_bytes(int nb) {
-    return (size_t)kMmaPos * (kMmaABlock + kMmaPad) + (size_t)kMmaPos * (2 * nb * 16 + kMmaPad);
+    return (size_t)kMmaPos * (kMmaM * 16 + kMmaPad) + (size_t)kMmaPos * (nb * 16 + kMmaPad);
 }
 
 // bounded wait: a broken pipeline traps (launch error) instead of hanging the GPU
@@ -1670,12 +1679,9 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes
     return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
            ((uint64_t)8 << 32) | (1ull << 46);
 }
-__device__ __forceinline__ void expand_store(uint32_t w, uint32_t dst, uint32_t kc_stride) {
-    uint32_t e[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) e[j] = (w >> j) & 0x01010101u;
-    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(e[0]), "r"(e[1]), "r"(e[2]), "r"(e[3]) : "memory");
-    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst + kc_stride), "r"(e[4]), "r"(e[5]), "r"(e[6]), "r"(e[7]) : "memory");
+__device__ __forceinline__ void expand_store(uint32_t w, uint32_t dst) {
+    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"((w << 1) & 0x22222222u), "r"(w & 0x22222222u),
+                 "r"((w >> 1) & 0x22222222u), "r"((w >> 2) & 0x22222222u) : "memory");
 }
 
 __global__ void __launch_bounds__(kMmaThreads, 1)
@@ -1723,7 +1729,18 @@ k_score_mma(const a3d_job_t* __restrict__ jobs, int H, int pitch, int tt_tiles, 
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s_tmem)), "r"(kMmaTmemCols));
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
     }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    if (warp < 4) {
+        // block scales: every byte of columns kMmaSfCol.. of the warp's 32 lanes = 0x7F (UE8M0 2^0)
+        const uint32_t one = 0x7F7F7F7Fu;
+#pragma unroll
+        for (int c = kMmaSfCol; c < kMmaTmemCols; c += 8)
+            asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};"
+                         ::"r"(s_tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)c), "r"(one) : "memory");
+        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+    }
     for (int m = tid; m < nt + nc; m += kMmaThreads) {
         const int32_t* b;
         if (m < nt) {
@@ -1747,7 +1764,7 @@ k_score_mma(const a3d_job_t* __restrict__ jobs, int H, int pitch, int tt_tiles, 
     const uint32_t tmem = s_tmem;
 
     // region = (hull of the target boxes) ∩ (hull of the candidate boxes), walked as one row-major
-    // sequence of word positions; a step = kMmaPos consecutive positions = kMmaPos MMAs
+    // sequence of word positions; a step = kMmaPos consecutive positions = kMmaPos / 2 MMAs
     const int ra = max(s_box[0], s_box[4]), rb = min(s_box[1], s_box[5]);
     const int ca = max(s_box[2], s_box[6]), ce = min(s_box[3], s_box[7]);
     int npos = 0, ncols = 1;
@@ -1758,32 +1775,31 @@ k_score_mma(const a3d_job_t* __restrict__ jobs, int H, int pitch, int tt_tiles, 
     const int nsteps = (npos + kMmaPos - 1) / kMmaPos;
     const uint32_t stage0 = smem_u32(stage_mem);
     const uint32_t stage_bytes = (uint32_t)mma_stage_bytes(nb);
-    const uint32_t b_off = (uint32_t)kMmaPos * (kMmaABlock + kMmaPad);
-    const uint32_t b_block = (uint32_t)(2 * nb * 16);
+    const uint32_t a_slot = (uint32_t)(kMmaM * 16 + kMmaPad), b_slot = (uint32_t)(nb * 16 + kMmaPad);
+    const uint32_t b_off = (uint32_t)kMmaPos * a_slot;
     const uint32_t bar0 = smem_u32(&s_bar[0]);
 
     if (warp < kMmaProducerWarps) {
         // ===== producers =====
-        // thread -> word (tid & 3) of the step, for the masks (tid >> 2) + 128 u: one position cursor per
-        // thread, a constant stage slot per (thread, u).  Loads run kMmaAhead steps ahead of the stores in
-        // a register ring (static indices through full unrolling).
+        // thread -> word q of the step, for the masks tid / kMmaPos + (kMmaProducers / kMmaPos) u: one
+        // position cursor per thread, a constant stage slot per (thread, u).  Loads run kMmaAhead steps
+        // ahead of the stores in a register ring (static indices through full unrolling).  Positions past
+        // the region load as zeros, so an odd last position pairs with a zero chunk.
         const int nmask = nt + nc;
+        const int npos2 = (npos + 1) & ~1;
         const int q = tid & (kMmaPos - 1);
         const uint32_t* src[kMmaItems];             // word (ra, ca) of this thread's masks
         uint32_t dst[kMmaItems];                    // byte offset of the mask's 16-byte row slot inside a stage
-        uint32_t kcs[kMmaItems];                    // distance of the second K chunk
         bool act[kMmaItems];
 #pragma unroll
         for (int u = 0; u < kMmaItems; ++u) {
-            const int m = (tid >> 2) + u * (kMmaProducers / kMmaPos);
+            const int m = tid / kMmaPos + u * (kMmaProducers / kMmaPos);
             act[u] = m < nmask;
             src[u] = act[u] ? s_ptr[m] + (size_t)ra * pitch + ca : nullptr;
-            const bool a_row = m < nt;
-            dst[u] = a_row ? (uint32_t)q * (kMmaABlock + kMmaPad) + (uint32_t)m * 16u
-                           : b_off + (uint32_t)q * (b_block + kMmaPad) + (uint32_t)(m - nt) * 16u;
-            kcs[u] = a_row ? (uint32_t)(kMmaM * 16) : (uint32_t)nb * 16u;
+            dst[u] = m < nt ? (uint32_t)q * a_slot + (uint32_t)m * 16u
+                            : b_off + (uint32_t)q * b_slot + (uint32_t)(m - nt) * 16u;
         }
-        // position of this thread's word in the step the load cursor is at: p = 4 k + q = row * ncols + col
+        // position of this thread's word in the step the load cursor is at: p = kMmaPos k + q = row * ncols + col
         const int dr = kMmaPos / ncols, dc = kMmaPos - dr * ncols;
         int p_ld = q, col = q % ncols;
         unsigned rowoff = (unsigned)((q / ncols) * pitch);
@@ -1792,7 +1808,7 @@ k_score_mma(const a3d_job_t* __restrict__ jobs, int H, int pitch, int tt_tiles, 
             const bool in = p_ld < npos;
 #pragma unroll
             for (int u = 0; u < kMmaItems; ++u)
-                if (act[u] && in) w[u] = __ldg(src[u] + o);
+                if (act[u]) w[u] = in ? __ldg(src[u] + o) : 0u;
             p_ld += kMmaPos;
             col += dc;
             rowoff += (unsigned)(dr * pitch);
@@ -1802,10 +1818,10 @@ k_score_mma(const a3d_job_t* __restrict__ jobs, int H, int pitch, int tt_tiles, 
         auto store_step = [&](int st, uint32_t parity, const uint32_t (&w)[kMmaItems]) {
             const uint32_t sa = stage0 + (uint32_t)st * stage_bytes;
             mbar_wait_bounded(bar0 + 8u * (uint32_t)(kMmaStages + st), parity ^ 1u);
-            if (p_st < npos) {
+            if (p_st < npos2) {
 #pragma unroll
                 for (int u = 0; u < kMmaItems; ++u)
-                    if (act[u]) expand_store(w[u], sa + dst[u], kcs[u]);
+                    if (act[u]) expand_store(w[u], sa + dst[u]);
             }
             p_st += kMmaPos;
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // generic-proxy stores -> async-proxy (MMA) reads
@@ -1816,7 +1832,7 @@ k_score_mma(const a3d_job_t* __restrict__ jobs, int H, int pitch, int tt_tiles, 
             mbar_arrive(bar0 + 8u * (uint32_t)st);
 #endif
         };
-        static_assert(kMmaAhead % kMmaStages == 0, "stage and phase of a step must be static in the unrolled loop");
+        static_assert(kMmaAhead % kMmaStages == 0, "the stage of a step must be static in the unrolled loop");
         uint32_t ring[kMmaAhead][kMmaItems];
 #pragma unroll
         for (int d = 0; d < kMmaAhead - 1; ++d)
@@ -1827,27 +1843,29 @@ k_score_mma(const a3d_job_t* __restrict__ jobs, int H, int pitch, int tt_tiles, 
                 const int k = k0 + d;
                 if (k < nsteps) {
                     if (k + kMmaAhead - 1 < nsteps) load_step(ring[(d + kMmaAhead - 1) % kMmaAhead]);
-                    store_step(d % kMmaStages, (uint32_t)((d / kMmaStages) & 1), ring[d]);
+                    store_step(d % kMmaStages, (uint32_t)((k / kMmaStages) & 1), ring[d]);
                 }
             }
         }
     } else if (lane == 0) {
         // ===== MMA issuer (one thread) =====
-        const uint32_t idesc = (2u << 4) | ((uint32_t)(nb >> 3) << 17) | ((uint32_t)(kMmaM >> 4) << 24);   // u8 x u8 -> s32, K-major
+        // e2m1 x e2m1 -> f32, UE8M0 block scales, K-major
+        const uint32_t idesc = (1u << 7) | (1u << 10) | ((uint32_t)(nb >> 3) << 17) | (1u << 23) | ((uint32_t)(kMmaM >> 4) << 24);
+        const uint32_t sfa = tmem + (uint32_t)kMmaSfCol, sfb = sfa + 128u;
         for (int k = 0; k < nsteps; ++k) {
             const int st = k % kMmaStages;
-            const int cw = min(kMmaPos, npos - k * kMmaPos);
+            const int nmma = (min(kMmaPos, npos - k * kMmaPos) + 1) >> 1;
             const uint32_t sa = stage0 + (uint32_t)st * stage_bytes, sb = sa + b_off;
             mbar_wait_bounded(bar0 + 8u * (uint32_t)st, (uint32_t)((k / kMmaStages) & 1));
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            for (int j = 0; j < cw; ++j) {
-                const uint64_t da = umma_desc(sa + (uint32_t)j * (kMmaABlock + kMmaPad), kMmaM * 16);
-                const uint64_t db = umma_desc(sb + (uint32_t)j * (b_block + kMmaPad), (uint32_t)nb * 16u);
+            for (int j = 0; j < nmma; ++j) {
+                const uint64_t da = umma_desc(sa + (uint32_t)(2 * j) * a_slot, a_slot);
+                const uint64_t db = umma_desc(sb + (uint32_t)(2 * j) * b_slot, b_slot);
                 const uint32_t acc = (k > 0 || j > 0) ? 1u : 0u;
                 asm volatile(
-                    "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                    "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-                    ::"r"(tmem), "l"(da), "l"(db), "r"(idesc), "r"(acc) : "memory");
+                    "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %6, 0;\n\t"
+                    "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.scale_vec::2X [%0], %1, %2, %3, [%4], [%5], p;\n\t}"
+                    ::"r"(tmem), "l"(da), "l"(db), "r"(idesc), "r"(sfa), "r"(sfb), "r"(acc) : "memory");
             }
             // arrives on the stage's empty barrier once these MMAs have read shared memory
             asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
@@ -1887,7 +1905,7 @@ k_score_mma(const a3d_job_t* __restrict__ jobs, int H, int pitch, int tt_tiles, 
                 for (int j = 0; j < 16; ++j) {
                     const int c = c0 + j;
                     if (c < nc) {
-                        const int inter = (int)v[j];
+                        const int inter = __float2int_rn(__uint_as_float(v[j]));   // an integer, at most 2^24
                         const int uni = pt + s_pc[c] - inter;
                         const float iou = __fdiv_rn((float)inter, (float)uni);
                         const unsigned long long key = make_key(iou, cb + c, inter, packed);
@@ -2869,9 +2887,10 @@ static int score_impl(int H, int W, const a3d_job_t* jobs, int n_jobs, int max_t
     // Three scoring kernels with identical results (A3D_SCORE_KERNEL = ldg | tma | mma forces one):
     //  * k_score ("ldg"): AND + popcount on the integer pipes, direct loads, per-warp regions — every SM
     //    works on every job, so it is the one for few or small jobs;
-    //  * k_score_mma ("mma"): tensor cores (tcgen05 kind::i8 on bit-expanded masks), one CTA per
+    //  * k_score_mma ("mma"): tensor cores (tcgen05 kind::mxf4 on bit-expanded masks), one CTA per
     //    (job, 128 targets, <= 240 candidates); its time is ~245 us per wave of CTAs almost regardless of
-    //    the candidate count.  Measured on B200 (tools/score_ab.py), 120 targets per job:
+    //    the candidate count.  Measured on B200 (tools/score_ab.py) with the earlier kind::i8 kernel (the
+    //    kind::mxf4 one is faster: 308 vs 1237 us on the first shape), 120 targets per job:
     //    180 candidates x 256 jobs 440 us vs 1232 us; x 64 jobs 251 vs 322; x 48 jobs 249 vs 245;
     //    720 candidates x 64 jobs 421 vs 1138; but 60 x 90 x 256 jobs 339 vs 355 and 60 x 45: 323 vs 204
     //    — hence the automatic choice below: enough CTAs to fill the SMs and big (target, candidate) tiles;
@@ -2883,7 +2902,9 @@ static int score_impl(int H, int W, const a3d_job_t* jobs, int n_jobs, int max_t
     if (mma_ctile > kMmaNMax) mma_ctile = kMmaNMax;
     const long long mma_blocks = (long long)n_jobs * ((max_tgt + kMmaM - 1) / kMmaM) * ((max_cand + mma_ctile - 1) / mma_ctile);
     const bool mma_auto = mma_blocks >= 60 && (long long)(max_tgt < kMmaM ? max_tgt : kMmaM) * mma_ctile >= 16384;
-    const bool use_mma = env_kernel ? !strcmp(env_kernel, "mma") : mma_auto;
+    // its f32 accumulators count exactly up to 2^24: larger frames always take k_score
+    const bool mma_exact = (long long)H * W <= (1LL << 24);
+    const bool use_mma = mma_exact && (env_kernel ? !strcmp(env_kernel, "mma") : mma_auto);
     if (use_mma) {
         // tensor-core scoring: CTA = (job, 128 targets, <= 240 candidates)
         const int ctile = mma_ctile;

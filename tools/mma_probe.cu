@@ -1,52 +1,59 @@
-// Stand-alone probe of tcgen05.mma kind::i8 (u8 x u8 -> s32) with hand-built shared-memory
-// descriptors in the no-swizzle K-major ("interleaved core matrix") layout, accumulator in TMEM,
-// read back with tcgen05.ld.32x32b.  Used to pin the descriptor fields before k_score_mma was
-// written (DESIGN.md §4).  Build: nvcc -gencode arch=compute_100a,code=sm_100a -o mma_probe mma_probe.cu
+// Stand-alone probe of tcgen05.mma kind::mxf4 (e2m1 x e2m1 -> f32, UE8M0 block scales) as k_score_mma
+// uses it: mask words expanded to nibbles (bit -> 0x2 = 1.0, 0 -> 0.0) in the no-swizzle K-major
+// layout [word position][row][16 B] with padded position slots, one MMA (K = 64) per two positions,
+// every scale byte 0x7F (= 1.0) in TMEM columns 256..511, accumulator in TMEM columns 0..255.
+//
+// It pins the instruction descriptor and the descriptor fields, and checks that the accumulator
+// counts exactly: every product is 0 or 1, so an f32 accumulator with a full 24-bit significand holds
+// every count below 2^24 exactly.  The contraction runs over 2^21 + 96 pixels and all 128 x N
+// accumulators are read at checkpoints past 2^14, 2^16, 2^20, 786 432 (= 1024 x 768) and 2^21,
+// against an integer popcount reference.  Rows: all ones, random at several densities, and a
+// candidate with one bit per 64-pixel block (adds 1 per MMA onto a large sum).
+//
+// Build: nvcc -gencode arch=compute_100a,code=sm_100a -O2 -Xcompiler -mpopcnt -o tools/mma_probe tools/mma_probe.cu
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <vector>
 #include <cuda_runtime.h>
 
 #define CK(x) do { cudaError_t e = (x); if (e != cudaSuccess) { printf("CUDA error %s at %s:%d\n", cudaGetErrorString(e), __FILE__, __LINE__); exit(2); } } while (0)
+
+constexpr int kM = 128;
+constexpr int kNMax = 240;
+constexpr int kPos = 8;                 // word positions per round = 4 MMAs
+constexpr int kPad = 16;                // as k_score_mma at 8 positions per stage: slots 16-byte aligned only
+constexpr int kWords = (1 << 16) + 3;   // words per mask row: 2^21 + 96 pixels (odd: a zero-filled tail chunk)
+constexpr int kChecks = 6;
+__constant__ int c_check[kChecks];      // word counts after which the accumulators are read
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
+    uint32_t ok, spins = 0;
     do {
         asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
                      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
+        if (!ok && ++spins > (1u << 24)) __trap();
     } while (!ok);
 }
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-    return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo >> 4) & 0x3FFF) << 16) |
-           ((uint64_t)((sbo >> 4) & 0x3FFF) << 32) | (1ull << 46);
+__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo) {
+    return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo >> 4) & 0x3FFF) << 16) | ((uint64_t)8 << 32) | (1ull << 46);
 }
 
-// A: [128][K] bytes row-major, B: [N][K] bytes row-major, D: [128][N] s32
-__global__ void __launch_bounds__(128) probe(const uint8_t* A, const uint8_t* B, int N, int K, int swap, int32_t* D) {
+// A: [128][kWords], B: [N][kWords] mask words; D: [kChecks][128][N] raw f32 accumulator bits
+__global__ void __launch_bounds__(128) probe(const uint32_t* A, const uint32_t* B, int N, uint32_t* D) {
     extern __shared__ __align__(1024) uint8_t smem[];
     __shared__ uint32_t tmem_base;
     __shared__ __align__(8) uint64_t bar;
-    const int nk = K / 32;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    uint8_t* sA = smem;
-    uint8_t* sB = smem + (size_t)nk * 2 * 128 * 16;
-    // layout per K=32 step: [kc(2)][rows][16 bytes]
-    for (int i = tid; i < 128 * K; i += 128) {
-        const int m = i / K, k = i % K;
-        sA[(size_t)(k / 32) * (2 * 128 * 16) + ((k % 32) / 16) * (128 * 16) + m * 16 + (k % 16)] = A[i];
-    }
-    for (int i = tid; i < N * K; i += 128) {
-        const int m = i / K, k = i % K;
-        sB[(size_t)(k / 32) * (2 * N * 16) + ((k % 32) / 16) * (N * 16) + m * 16 + (k % 16)] = B[i];
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    const uint32_t slotA = kM * 16 + kPad, slotB = (uint32_t)N * 16 + kPad;
+    const uint32_t sA = smem_u32(smem), sB = sA + kPos * slotA;
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base)), "r"(256));
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base)), "r"(512));
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
     }
     if (tid == 0) {
@@ -57,75 +64,140 @@ __global__ void __launch_bounds__(128) probe(const uint8_t* A, const uint8_t* B,
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = tmem_base;
-    if (tid == 0) {
-        const uint32_t idesc = (2u << 4) | ((uint32_t)(N >> 3) << 17) | ((128u >> 4) << 24);
-        for (int k = 0; k < nk; ++k) {
-            const uint32_t a0 = smem_u32(sA + (size_t)k * 2 * 128 * 16), b0 = smem_u32(sB + (size_t)k * 2 * N * 16);
-            const uint32_t lboA = 128 * 16, lboB = N * 16, sbo = 128;
-            const uint64_t da = swap ? make_desc(a0, sbo, lboA) : make_desc(a0, lboA, sbo);
-            const uint64_t db = swap ? make_desc(b0, sbo, lboB) : make_desc(b0, lboB, sbo);
-            const uint32_t acc = k > 0 ? 1u : 0u;
-            asm volatile(
-                "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-                ::"r"(tmem), "l"(da), "l"(db), "r"(idesc), "r"(acc) : "memory");
-        }
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(&bar)) : "memory");
-    }
-    mbar_wait(smem_u32(&bar), 0);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    for (int c0 = 0; c0 < N; c0 += 16) {
-        uint32_t r[16];
-        const uint32_t taddr = tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0;
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                     : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                       "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                     : "r"(taddr));
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        for (int j = 0; j < 16; ++j) D[(size_t)(warp * 32 + lane) * N + c0 + j] = (int32_t)r[j];
+    {   // scale factors: 0x7F (UE8M0 2^0) in every byte of columns 256..511 of all 128 lanes
+        const uint32_t one = 0x7F7F7F7Fu;
+        for (int c = 256; c < 512; c += 8)
+            asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};"
+                         ::"r"(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)c), "r"(one) : "memory");
+        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(256));
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    // e2m1 x e2m1 -> f32, UE8M0 scales, K-major, M = 128
+    const uint32_t idesc = (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | (1u << 23) | ((uint32_t)(kM >> 4) << 24);
+    int chk = 0;
+    uint32_t phase = 0;
+    for (int w0 = 0; w0 < kWords; w0 += kPos) {
+        const int nw = min(kPos, kWords - w0);
+        for (int i = tid; i < (kM + N) * kPos; i += 128) {
+            const int m = i / kPos, q = i % kPos;
+            const uint32_t w = q < nw ? (m < kM ? A[(size_t)m * kWords + w0 + q] : B[(size_t)(m - kM) * kWords + w0 + q]) : 0u;
+            const uint32_t dst = m < kM ? sA + q * slotA + m * 16 : sB + q * slotB + (m - kM) * 16;
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"((w << 1) & 0x22222222u), "r"(w & 0x22222222u),
+                         "r"((w >> 1) & 0x22222222u), "r"((w >> 2) & 0x22222222u) : "memory");
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        __syncthreads();
+        if (tid == 0) {
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            for (int j = 0; j < (nw + 1) / 2; ++j) {
+                const uint64_t da = make_desc(sA + 2 * j * slotA, slotA);
+                const uint64_t db = make_desc(sB + 2 * j * slotB, slotB);
+                const uint32_t acc = (w0 > 0 || j > 0) ? 1u : 0u;
+                asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %6, 0;\n\t"
+                             "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.scale_vec::2X [%0], %1, %2, %3, [%4], [%5], p;\n\t}"
+                             ::"r"(tmem), "l"(da), "l"(db), "r"(idesc), "r"(tmem + 256u), "r"(tmem + 384u), "r"(acc) : "memory");
+            }
+            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(&bar)) : "memory");
+        }
+        mbar_wait(smem_u32(&bar), phase);
+        phase ^= 1u;
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        if (chk < kChecks && w0 + nw == c_check[chk]) {
+            for (int c0 = 0; c0 < N; c0 += 16) {
+                uint32_t r[16];
+                asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                             : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+                               "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                             : "r"(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0));
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                for (int j = 0; j < 16; ++j) D[((size_t)chk * kM + warp * 32 + lane) * N + c0 + j] = r[j];
+            }
+            ++chk;
+        }
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        __syncthreads();                                   // smem and accumulator reads done before the next round
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    }
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
 }
 
 int main() {
-    const int Ns[] = {16, 96, 192, 240};
-    const int K = 128;
-    int bad_total = 0;
-    for (int swap = 0; swap < 2; ++swap)
-        for (int N : Ns) {
-            std::vector<uint8_t> A(128 * K), B(N * K);
-            uint32_t s = 12345u + N;
-            auto rnd = [&]() { s = s * 1664525u + 1013904223u; return (s >> 16) & 1u; };
-            for (auto& v : A) v = (uint8_t)rnd();
-            for (auto& v : B) v = (uint8_t)rnd();
-            std::vector<int32_t> ref(128 * N, 0), out(128 * N, -1);
-            for (int m = 0; m < 128; ++m)
-                for (int n = 0; n < N; ++n) {
-                    int acc = 0;
-                    for (int k = 0; k < K; ++k) acc += A[m * K + k] * B[n * K + k];
-                    ref[m * N + n] = acc;
-                }
-            uint8_t *dA, *dB; int32_t* dD;
-            CK(cudaMalloc(&dA, A.size())); CK(cudaMalloc(&dB, B.size())); CK(cudaMalloc(&dD, out.size() * 4));
-            CK(cudaMemcpy(dA, A.data(), A.size(), cudaMemcpyHostToDevice));
-            CK(cudaMemcpy(dB, B.data(), B.size(), cudaMemcpyHostToDevice));
-            CK(cudaMemset(dD, 0xff, out.size() * 4));
-            const size_t smem = (size_t)(K / 32) * 2 * 16 * (128 + N);
-            CK(cudaFuncSetAttribute(probe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            probe<<<1, 128, smem>>>(dA, dB, N, K, swap, dD);
-            cudaError_t e = cudaDeviceSynchronize();
-            if (e != cudaSuccess) { printf("swap=%d N=%d: kernel error %s\n", swap, N, cudaGetErrorString(e)); return 3; }
-            CK(cudaMemcpy(out.data(), dD, out.size() * 4, cudaMemcpyDeviceToHost));
-            int bad = 0;
-            for (size_t i = 0; i < out.size(); ++i) bad += out[i] != ref[i];
-            printf("swap=%d N=%d: %d / %zu mismatches; D[0][0..3] = %d %d %d %d (ref %d %d %d %d); D[1][0]=%d (ref %d) D[127][N-1]=%d (ref %d)\n",
-                   swap, N, bad, out.size(), out[0], out[1], out[2], out[3], ref[0], ref[1], ref[2], ref[3],
-                   out[N], ref[N], out[127 * N + N - 1], ref[127 * N + N - 1]);
-            if (swap == 0) bad_total += bad;
-            cudaFree(dA); cudaFree(dB); cudaFree(dD);
+    // checkpoints (words): just past 2^14 and 2^16 pixels, then 786 432, 2^20, 2^20 + 256 and 2^21 + 96 pixels
+    const int checks[kChecks] = {(1 << 9) + 8, (1 << 11) + 8, 24576, (1 << 15), (1 << 15) + 8, kWords};
+    CK(cudaMemcpyToSymbol(c_check, checks, sizeof(checks)));
+    uint64_t s = 0x9E3779B97F4A7C15ull;
+    auto rnd = [&]() { s ^= s << 13; s ^= s >> 7; s ^= s << 17; return (uint32_t)s; };
+    auto word = [&](int kind) -> uint32_t {   // density: 1, 1/2, 1/4, 3/4, 31/32
+        switch (kind) {
+            case 0: return 0xFFFFFFFFu;
+            case 1: return rnd();
+            case 2: return rnd() & rnd();
+            case 3: return rnd() | rnd();
+            default: return ~(rnd() & rnd() & rnd() & rnd() & rnd());
         }
-    printf(bad_total == 0 ? "PROBE OK (lbo = K-chunk stride, sbo = 8-row group stride)\n" : "PROBE MISMATCH\n");
-    return 0;
+    };
+    std::vector<uint32_t> A((size_t)kM * kWords), B((size_t)kNMax * kWords);
+    for (int m = 0; m < kM; ++m)
+        for (int w = 0; w < kWords; ++w) A[(size_t)m * kWords + w] = word(m % 5);
+    for (int n = 0; n < kNMax; ++n)
+        for (int w = 0; w < kWords; ++w) {
+            uint32_t v = word((n + 1) % 6 == 5 ? 0 : (n % 5));
+            if (n % 6 == 5) v = (w & 1) ? 0u : (1u << (w % 31));   // one bit per 64 pixels
+            B[(size_t)n * kWords + w] = v;
+        }
+    // integer reference at every checkpoint
+    std::vector<int64_t> ref((size_t)kChecks * kM * kNMax);
+    for (int m = 0; m < kM; ++m)
+        for (int n = 0; n < kNMax; ++n) {
+            const uint32_t* a = &A[(size_t)m * kWords];
+            const uint32_t* b = &B[(size_t)n * kWords];
+            int64_t acc = 0;
+            int c = 0;
+            for (int w = 0; w < kWords; ++w) {
+                acc += __builtin_popcount(a[w] & b[w]);
+                if (w + 1 == checks[c]) ref[((size_t)c++ * kM + m) * kNMax + n] = acc;
+            }
+        }
+    uint32_t *dA, *dB, *dD;
+    CK(cudaMalloc(&dA, A.size() * 4)); CK(cudaMalloc(&dB, B.size() * 4));
+    CK(cudaMalloc(&dD, (size_t)kChecks * kM * kNMax * 4));
+    CK(cudaMemcpy(dA, A.data(), A.size() * 4, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(dB, B.data(), B.size() * 4, cudaMemcpyHostToDevice));
+    int bad_total = 0;
+    for (int N : {16, 192, 240}) {
+        const size_t smem = (size_t)kPos * (kM * 16 + kPad) + (size_t)kPos * (N * 16 + kPad);
+        CK(cudaFuncSetAttribute(probe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CK(cudaMemset(dD, 0xff, (size_t)kChecks * kM * N * 4));
+        probe<<<1, 128, smem>>>(dA, dB, N, dD);
+        cudaError_t e = cudaDeviceSynchronize();
+        if (e != cudaSuccess) { printf("N=%d: kernel error %s\n", N, cudaGetErrorString(e)); return 3; }
+        std::vector<uint32_t> out((size_t)kChecks * kM * N);
+        CK(cudaMemcpy(out.data(), dD, out.size() * 4, cudaMemcpyDeviceToHost));
+        for (int c = 0; c < kChecks; ++c) {
+            int bad = 0;
+            int64_t vmax = 0, first_bad_ref = -1;
+            float first_bad_got = 0.f;
+            for (int m = 0; m < kM; ++m)
+                for (int n = 0; n < N; ++n) {
+                    const int64_t r = ref[((size_t)c * kM + m) * kNMax + n];
+                    float f;
+                    memcpy(&f, &out[((size_t)c * kM + m) * N + n], 4);
+                    vmax = r > vmax ? r : vmax;
+                    if ((double)f != (double)r) {
+                        if (!bad) { first_bad_ref = r; first_bad_got = f; }
+                        ++bad;
+                    }
+                }
+            printf("N=%3d after %8d pixels: %5d / %d accumulators wrong, largest count %lld", N, checks[c] * 32, bad, kM * N,
+                   (long long)vmax);
+            if (bad) printf("  (first: got %.1f, want %lld)", first_bad_got, (long long)first_bad_ref);
+            printf("\n");
+            bad_total += bad;
+        }
+    }
+    printf(bad_total == 0 ? "PROBE OK: kind::mxf4 counts exactly up to 2^21 + 96 (idesc e2m1 x e2m1 -> f32, UE8M0 = 0x7F)\n"
+                          : "PROBE MISMATCH\n");
+    return bad_total != 0;
 }

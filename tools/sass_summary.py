@@ -10,7 +10,7 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "articulation3d_b200", "csrc", "liba3d.so")
 tag = sys.argv[1] if len(sys.argv) > 1 else "r2"
-WATCH = ["UTCIMMA", "UTCHMMA", "UTCQMMA", "LDTM", "STTM", "UTCBAR", "UTMALDG", "UTMASTG", "UBLKCP", "SYNCS", "POPC", "ATOMS", "RED",
+WATCH = ["UTCOMMA", "UTCIMMA", "UTCHMMA", "UTCQMMA", "LDTM", "STTM", "UTCBAR", "UTMALDG", "UTMASTG", "UBLKCP", "SYNCS", "POPC", "ATOMS", "RED",
          "ATOMG", "MUFU.RCP", "FFMA", "FFMA2", "DFMA", "DMUL", "DADD", "LOP3", "IMAD", "SHF", "FSETP", "LDS", "STS",
          "LDG", "STG", "REDUX", "BAR", "ACQBULK", "PREEXIT"]
 
@@ -48,7 +48,7 @@ usage = {}
 for m in re.finditer(r"Function (\S+):\s*\n\s*REG:(\d+) .*?SHARED:(\d+)", res):
     usage[m.group(1)] = (int(m.group(2)), int(m.group(3)))
 lines = [f"# SASS mnemonic counts per kernel of articulation3d_b200/csrc/liba3d.so (cuobjdump -sass, sm_100a), {tag}",
-         "# UTCIMMA = tcgen05.mma kind::i8, LDTM = tcgen05.ld, UTCBAR = tcgen05.commit, UTMALDG = TMA tensor load, "
+         "# UTCOMMA = tcgen05.mma kind::mxf4, LDTM = tcgen05.ld, UTCBAR = tcgen05.commit, UTMALDG = TMA tensor load, "
          "ATOMS/RED = shared / global atomics", ""]
 for k, c in kernels.items():
     reg, sh = usage.get(k, (None, None))
