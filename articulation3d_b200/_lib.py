@@ -38,12 +38,22 @@ JOB_DTYPE = np.dtype([
 ], align=True)
 assert JOB_DTYPE.itemsize == 72, JOB_DTYPE.itemsize
 
+# a3d_layer_t / a3d_segment_t (a3d_render) as numpy structured dtypes, C layout
+LAYER_FILL, LAYER_OUTLINE = 0, 1
+LAYER_DTYPE = np.dtype([("mask", "<i4"), ("kind", "<i4"), ("rgba", "u1", (4,))])
+SEGMENT_DTYPE = np.dtype([("x0", "<i4"), ("y0", "<i4"), ("x1", "<i4"), ("y1", "<i4"), ("radius", "<i4"),
+                          ("rgb", "u1", (3,)), ("pad", "u1")])
+assert LAYER_DTYPE.itemsize == 12 and SEGMENT_DTYPE.itemsize == 24
+RENDER_MAX_SIDE = 16384      # A3D_RENDER_MAX_SIDE
+RENDER_MAX_COORD = 1 << 14   # |segment coordinate| limit of a3d_render
+RENDER_MAX_RADIUS = 256
+
 # every symbol include/a3d.h declares
 EXPORTS = (
     "a3d_version", "a3d_last_error_string", "a3d_pitch_words", "a3d_project_max_tile",
     "a3d_pack_masks", "a3d_mask_meta", "a3d_project", "a3d_score", "a3d_pass", "a3d_emit_masks",
     "a3d_rle_to_bits", "a3d_plane_offsets", "a3d_plan_tiles", "a3d_host_quat_to_xform", "a3d_fetch_host_block", "a3d_upload_masks", "a3d_host_rle_counts",
-    "a3d_rle_count_runs", "a3d_bits_to_rle", "a3d_host_rle_strings",
+    "a3d_rle_count_runs", "a3d_bits_to_rle", "a3d_host_rle_strings", "a3d_render",
 )
 
 _lib = None
@@ -106,6 +116,8 @@ def load():
     lib.a3d_bits_to_rle.argtypes = [vp, vp, i64, i32, i32, vp, vp, vp]
     lib.a3d_plane_offsets.restype = C.c_int
     lib.a3d_plane_offsets.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp, vp]
+    lib.a3d_render.restype = C.c_int
+    lib.a3d_render.argtypes = [vp, i64, i32, i32, i32, vp, vp, i64, vp, vp, vp, vp, vp, vp]
     _lib = lib
     return lib
 

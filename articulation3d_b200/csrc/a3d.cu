@@ -3065,3 +3065,290 @@ int a3d_plane_offsets(const float* depth, const float* rays, int H, int W, const
 }
 
 }  // extern "C"
+
+// ---------------------------------------------------------------------------
+// render (a3d_render): masks and segments composited over the frames' backgrounds into RGB frames.
+// One CTA per (frame, band of rows).  The band's bytes are contiguous in the background and in `out`,
+// so they are staged in shared memory with 16-byte copies (bytes where the two addresses disagree modulo
+// 16), the frame's list entries that touch the band are culled into shared memory (a pass of up to
+// kRenderCap layers, then segments, at a time, in list order), and every thread composites whole packed
+// words: 32 pixels of one row per work item.  HBM traffic: the band's background bytes, its output bytes
+// and the words of the layers inside their boxes.
+// ---------------------------------------------------------------------------
+constexpr int kRenderThreads = 256;
+constexpr int kRenderCap = kRenderThreads;      // list entries culled per pass: one per thread
+constexpr int kRenderStageBytes = 32768;        // target size of a band's RGB staging
+
+struct RenderSeg {                              // a culled segment with its box clipped to the band
+    int x0, y0, x1, y1, r;
+    uint32_t rgb;
+    int bx0, bx1, by0, by1;
+};
+
+// block-wide copy of n bytes: 16-byte pieces when dst and src agree modulo 16, single bytes otherwise
+__device__ __forceinline__ void render_copy(uint8_t* dst, const uint8_t* src, int64_t n) {
+    const int t = threadIdx.x;
+    if ((((uintptr_t)dst ^ (uintptr_t)src) & 15) == 0) {
+        int64_t head = (16 - ((uintptr_t)dst & 15)) & 15;
+        if (head > n) head = n;
+        if (t < head) dst[t] = src[t];
+        const int64_t n16 = (n - head) >> 4;
+        uint4* d4 = (uint4*)(dst + head);
+        const uint4* s4 = (const uint4*)(src + head);
+        for (int64_t i = t; i < n16; i += 4 * kRenderThreads) {       // four loads in flight before the stores
+            uint4 v[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u)
+                if (i + u * kRenderThreads < n16) v[u] = s4[i + u * kRenderThreads];
+#pragma unroll
+            for (int u = 0; u < 4; ++u)
+                if (i + u * kRenderThreads < n16) d4[i + u * kRenderThreads] = v[u];
+        }
+        for (int64_t i = head + (n16 << 4) + t; i < n; i += kRenderThreads) dst[i] = src[i];
+    } else {
+        for (int64_t i = t; i < n; i += kRenderThreads) dst[i] = src[i];
+    }
+}
+
+// ordered block-wide compaction: the slot of this thread's entry among the kept ones; *total = kept count
+__device__ __forceinline__ int render_rank(bool keep, int* s_warp, int* total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned b = __ballot_sync(0xffffffffu, keep);
+    if (lane == 0) s_warp[warp] = __popc(b);
+    __syncthreads();
+    int base = 0, sum = 0;
+#pragma unroll
+    for (int w = 0; w < kRenderThreads / 32; ++w) {
+        const int c = s_warp[w];
+        base += w < warp ? c : 0;
+        sum += c;
+    }
+    *total = sum;
+    __syncthreads();
+    return base + __popc(b & ((1u << lane) - 1u));
+}
+
+// exact: squared distance of pixel (x, y) to the closed segment <= r^2, in int64 (|coordinates| <= 2^14, r <= 256)
+__device__ __forceinline__ bool render_seg_hit(const RenderSeg& s, int x, int y) {
+    const int64_t dx = s.x1 - s.x0, dy = s.y1 - s.y0, qx = x - s.x0, qy = y - s.y0;
+    const int64_t r2 = (int64_t)s.r * s.r;
+    const int64_t t = qx * dx + qy * dy, L = dx * dx + dy * dy;
+    if (t <= 0) return qx * qx + qy * qy <= r2;
+    if (t >= L) {
+        const int64_t ex = x - s.x1, ey = y - s.y1;
+        return ex * ex + ey * ey <= r2;
+    }
+    const int64_t c = qx * dy - qy * dx;
+    return c * c <= r2 * L;
+}
+
+// float64 reciprocal of a nonzero integer and square root of v >= 0 from the single-precision MUFU estimates and
+// two Newton steps: no IEEE slow-path subroutine (whose calling convention spills the kernel's live registers)
+__device__ __forceinline__ double render_rcp(double x) {
+    double r = (double)__fdividef(1.0f, (float)x);
+    r = r * (2.0 - x * r);
+    return r * (2.0 - x * r);
+}
+
+__device__ __forceinline__ double render_sqrt(double v) {
+    if (v <= 0.0) return 0.0;
+    double y = (double)rsqrtf((float)v);
+    y = y * (1.5 - 0.5 * v * y * y);
+    y = y * (1.5 - 0.5 * v * y * y);
+    return v * y;
+}
+
+// The pixels of row y within distance r of the segment form one interval (the capsule is convex).  Its ends,
+// estimated in float64 as the hull of the two end discs and the strip beside the segment; the caller decides
+// every pixel within one pixel of the estimate exactly, so only the estimate's error (far below a pixel) has
+// to be covered.  false: the row misses the capsule.
+__device__ __forceinline__ bool render_seg_row(const RenderSeg& s, int y, double* lo, double* hi) {
+    const double r = s.r, x0 = s.x0, x1 = s.x1;
+    double a = 1e30, b = -1e30;
+    const double h0 = r * r - (double)(y - s.y0) * (y - s.y0), h1 = r * r - (double)(y - s.y1) * (y - s.y1);
+    if (h0 >= 0) { const double w = render_sqrt(h0); a = fmin(a, x0 - w); b = fmax(b, x0 + w); }
+    if (h1 >= 0) { const double w = render_sqrt(h1); a = fmin(a, x1 - w); b = fmax(b, x1 + w); }
+    const int64_t idx = s.x1 - s.x0, idy = s.y1 - s.y0, iry = y - s.y0;
+    const int64_t iL = idx * idx + idy * idy;
+    if (iL > 0) {
+        const double dx = (double)idx, dy = (double)idy, ry = (double)iry, L = (double)iL;
+        double sa = -1e30, sb = 1e30;
+        bool ok = true;
+        if (idy != 0) {                          // |(x - x0) dy - ry dx| <= r sqrt(L)
+            const double idy_r = render_rcp(dy);
+            const double c = x0 + ry * dx * idy_r, w = r * render_sqrt(L) * fabs(idy_r);
+            sa = c - w;
+            sb = c + w;
+        } else {
+            ok = (iry * idx) * (iry * idx) <= (int64_t)s.r * s.r * iL;
+        }
+        if (idx != 0) {                          // 0 <= (x - x0) dx + ry dy <= L
+            const double idx_r = render_rcp(dx);
+            const double t0 = x0 - ry * dy * idx_r, t1 = x0 + (L - ry * dy) * idx_r;
+            sa = fmax(sa, fmin(t0, t1));
+            sb = fmin(sb, fmax(t0, t1));
+        } else {
+            ok = ok && iry * idy >= 0 && iry * idy <= iL;
+        }
+        if (ok && sa <= sb + 1e-6) { a = fmin(a, sa); b = fmax(b, sb); }
+    }
+    *lo = a;
+    *hi = b;
+    return a <= b;
+}
+
+__device__ __forceinline__ uint8_t render_blend(uint32_t c, uint32_t o, uint32_t a) {
+    return (uint8_t)((c * a + o * (255u - a) + 127u) / 255u);
+}
+
+__global__ void __launch_bounds__(kRenderThreads, 4)
+k_render(const uint8_t* __restrict__ bg, int64_t bg_stride, int f0, int H, int W, int pitch, int band_rows,
+         const uint32_t* __restrict__ bits, const int32_t* __restrict__ bbox, int64_t n_masks,
+         const a3d_layer_t* __restrict__ layers, const int64_t* __restrict__ layer_begin,
+         const a3d_segment_t* __restrict__ segs, const int64_t* __restrict__ seg_begin, uint8_t* __restrict__ out) {
+    extern __shared__ uint4 s_dyn[];
+    __shared__ int4 s_lay[kRenderCap];            // {mask | outline << 31, rgba, rows lo | hi << 16, words lo | hi << 16}
+    __shared__ RenderSeg s_seg[kRenderCap];
+    __shared__ int s_warp[kRenderThreads / 32];
+    const int f = f0 + blockIdx.y;
+    const int r0 = blockIdx.x * band_rows, r1 = min(H, r0 + band_rows);
+    const int64_t row_bytes = (int64_t)W * 3;
+    const int64_t nbytes = (r1 - r0) * row_bytes;
+    uint8_t* o = out + ((int64_t)f * H + r0) * row_bytes;
+    uint8_t* stage = (uint8_t*)s_dyn + ((uintptr_t)o & 15);        // same phase as `out`: aligned write-out
+    render_copy(stage, bg + (int64_t)f * bg_stride + r0 * row_bytes, nbytes);
+    const int nw = (W + 31) >> 5;
+    const int items = (r1 - r0) * nw;
+    int64_t li = layer_begin[f], si = seg_begin[f];
+    const int64_t le = layer_begin[f + 1], se = seg_begin[f + 1];
+    while (li < le || si < se) {
+        int nl = 0, ns = 0;
+        if (li < le) {
+            const int64_t k = li + threadIdx.x;
+            bool keep = false;
+            int4 e = make_int4(0, 0, 0, 0);
+            if (k < le) {
+                const a3d_layer_t L = layers[k];
+                if (L.mask >= 0 && L.mask < n_masks) {
+                    int rmin = 0, rmax = H - 1, wmin = 0, wmax = nw - 1;
+                    if (bbox) {
+                        const int4 b = ((const int4*)bbox)[L.mask];
+                        rmin = max(b.x, 0); rmax = min(b.y, H - 1); wmin = max(b.z, 0); wmax = min(b.w, nw - 1);
+                    }
+                    rmin = max(rmin, r0);
+                    rmax = min(rmax, r1 - 1);
+                    keep = rmin <= rmax && wmin <= wmax;
+                    const uint32_t rgba = L.rgba[0] | (uint32_t)L.rgba[1] << 8 | (uint32_t)L.rgba[2] << 16 |
+                                          (uint32_t)L.rgba[3] << 24;
+                    e = make_int4(L.mask | (L.kind == A3D_LAYER_OUTLINE ? (int)0x80000000u : 0), (int)rgba,
+                                  rmin | rmax << 16, wmin | wmax << 16);
+                }
+            }
+            const int slot = render_rank(keep, s_warp, &nl);
+            if (keep) s_lay[slot] = e;
+            li += kRenderCap;
+        }
+        if (li >= le && si < se) {
+            const int64_t k = si + threadIdx.x;
+            bool keep = false;
+            a3d_segment_t S{};
+            int bx0 = 0, bx1 = -1, by0 = 0, by1 = -1;
+            if (k < se) {
+                S = segs[k];
+                bx0 = max(0, min(S.x0, S.x1) - S.radius);
+                bx1 = min(W - 1, max(S.x0, S.x1) + S.radius);
+                by0 = max(r0, min(S.y0, S.y1) - S.radius);
+                by1 = min(r1 - 1, max(S.y0, S.y1) + S.radius);
+                keep = bx0 <= bx1 && by0 <= by1;
+            }
+            const int slot = render_rank(keep, s_warp, &ns);
+            if (keep) {
+                RenderSeg& e = s_seg[slot];
+                e.x0 = S.x0; e.y0 = S.y0; e.x1 = S.x1; e.y1 = S.y1; e.r = S.radius;
+                e.rgb = S.rgb[0] | (uint32_t)S.rgb[1] << 8 | (uint32_t)S.rgb[2] << 16;
+                e.bx0 = bx0; e.bx1 = bx1; e.by0 = by0; e.by1 = by1;
+            }
+            si += kRenderCap;
+        }
+        __syncthreads();
+        for (int it = threadIdx.x; it < items; it += kRenderThreads) {
+            const int rr = it / nw, j = it - rr * nw, y = r0 + rr;
+            uint8_t* px = stage + rr * row_bytes + j * 96;
+            const uint32_t valid = rle_valid(j, W);
+            for (int k = 0; k < nl; ++k) {
+                const int4 e = s_lay[k];
+                if (y < (e.z & 0xffff) || y > (e.z >> 16) || j < (e.w & 0xffff) || j > (e.w >> 16)) continue;
+                const uint32_t* mb = bits + ((int64_t)(e.x & 0x7fffffff) * H + y) * pitch;
+                uint32_t cov = mb[j] & valid;
+                if (!cov) continue;
+                if (e.x < 0) {                     // outline: set pixels with an unset 4-neighbour
+                    const uint32_t up = y > 0 ? mb[j - pitch] : 0u;
+                    const uint32_t dn = y + 1 < H ? mb[j + pitch] : 0u;
+                    const uint32_t lw = j > 0 ? mb[j - 1] : 0u;
+                    const uint32_t rw = j + 1 < nw ? mb[j + 1] : 0u;
+                    const uint32_t left = (cov << 1) | (lw >> 31), right = (cov >> 1) | (rw << 31);
+                    cov &= ~(up & dn & left & right);
+                }
+                const uint32_t c0 = e.y & 255, c1 = (e.y >> 8) & 255, c2 = (e.y >> 16) & 255, a = (uint32_t)e.y >> 24;
+                while (cov) {
+                    const int i = __ffs(cov) - 1;
+                    cov &= cov - 1;
+                    uint8_t* p = px + 3 * i;
+                    p[0] = render_blend(c0, p[0], a);
+                    p[1] = render_blend(c1, p[1], a);
+                    p[2] = render_blend(c2, p[2], a);
+                }
+            }
+            const int xa = 32 * j, xb = min(W, xa + 32) - 1;
+            for (int k = 0; k < ns; ++k) {
+                const RenderSeg s = s_seg[k];
+                if (y < s.by0 || y > s.by1 || xb < s.bx0 || xa > s.bx1) continue;
+                double lo, hi;
+                if (!render_seg_row(s, y, &lo, &hi)) continue;
+                const int xs = max(max(xa, s.bx0), (int)floor(fmax(lo, -1e9)) - 1);
+                const int xe = min(min(xb, s.bx1), (int)ceil(fmin(hi, 1e9)) + 1);
+                for (int x = xs; x <= xe; ++x) {
+                    if (!render_seg_hit(s, x, y)) continue;
+                    uint8_t* p = px + 3 * (x - xa);
+                    p[0] = s.rgb & 255;
+                    p[1] = (s.rgb >> 8) & 255;
+                    p[2] = (s.rgb >> 16) & 255;
+                }
+            }
+        }
+        __syncthreads();
+    }
+    __syncthreads();
+    render_copy(o, stage, nbytes);
+}
+
+extern "C" {
+
+int a3d_render(const uint8_t* background, int64_t bg_frame_stride, int n_frames, int H, int W,
+               const uint32_t* bits, const int32_t* bbox, int64_t n_masks,
+               const a3d_layer_t* layers, const int64_t* layer_begin,
+               const a3d_segment_t* segs, const int64_t* seg_begin, uint8_t* out, void* stream) {
+    if (n_frames < 0 || H <= 0 || W <= 0 || n_masks < 0 || bg_frame_stride < 0)
+        return fail(A3D_EINVAL, "a3d_render: bad shape n_frames=%d %dx%d n_masks=%lld stride=%lld", n_frames, H, W,
+                    (long long)n_masks, (long long)bg_frame_stride);
+    if (H > A3D_RENDER_MAX_SIDE || W > A3D_RENDER_MAX_SIDE)
+        return fail(A3D_ELIMIT, "a3d_render: %dx%d frame exceeds %d pixels a side", H, W, A3D_RENDER_MAX_SIDE);
+    if (n_frames == 0) return A3D_OK;
+    if (!background || !layer_begin || !seg_begin || !out || (n_masks > 0 && !bits))
+        return fail(A3D_EINVAL, "a3d_render: null pointer");
+    int band_rows = kRenderStageBytes / (3 * W);
+    band_rows = band_rows < 1 ? 1 : (band_rows > H ? H : band_rows);
+    const int smem = band_rows * 3 * W + 16;
+    A3D_CUDA_TRY(cudaFuncSetAttribute(k_render, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    const unsigned bands = (unsigned)((H + band_rows - 1) / band_rows);
+    for (int f0 = 0; f0 < n_frames; f0 += 65535) {
+        const unsigned nf = (unsigned)(n_frames - f0 < 65535 ? n_frames - f0 : 65535);
+        k_render<<<dim3(bands, nf), kRenderThreads, smem, (cudaStream_t)stream>>>(
+            background, bg_frame_stride, f0, H, W, pitch_words(W), band_rows, bits, bbox, n_masks, layers, layer_begin,
+            segs, seg_begin, out);
+        A3D_CUDA_TRY(cudaGetLastError());
+    }
+    return A3D_OK;
+}
+
+}  // extern "C"

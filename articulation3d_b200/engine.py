@@ -763,3 +763,83 @@ def plane_offsets(pool: MaskPool, inst_mask: torch.Tensor, normals: torch.Tensor
                                          normals.data_ptr(), n, off.data_ptr(), cnt.data_ptr(), _stream_ptr()),
                    "a3d_plane_offsets")
     return off, cnt
+
+
+def _render_begin(begin, n_items: int, name: str) -> np.ndarray:
+    b = np.asarray(begin)
+    if b.ndim != 1 or len(b) < 1 or b.dtype.kind not in "iu":
+        raise ValueError(f"{name} must be a 1-D integer array of n_frames + 1 offsets")
+    b = b.astype(np.int64)
+    if b[0] != 0 or np.any(np.diff(b) < 0) or b[-1] != n_items:
+        raise ValueError(f"{name} must rise monotonically from 0 to the list length {n_items}")
+    return b
+
+
+def render(pool: MaskPool | None, layers: np.ndarray, layer_begin, segs: np.ndarray, seg_begin,
+           background: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+    """Frames of masks and segments composited over a background on the device (``a3d_render``).
+
+    ``layers`` (``_lib.LAYER_DTYPE``) and ``segs`` (``_lib.SEGMENT_DTYPE``) are host arrays; frame f draws
+    ``layers[layer_begin[f]:layer_begin[f+1]]`` (fills and outlines of ``pool`` masks, blended), then its
+    segments (opaque).  ``background`` is one (H, W, 3) uint8 image for all frames or (n_frames, H, W, 3), on the
+    device.  Returns (n_frames, H, W, 3) uint8 RGB on the background's device (``out`` if given).  Everything
+    from outside is checked before the launch: ValueError for bad lists, limits or shapes."""
+    if not isinstance(layers, np.ndarray) or layers.dtype != _lib.LAYER_DTYPE or layers.ndim != 1:
+        raise ValueError("layers must be a 1-D numpy array of _lib.LAYER_DTYPE")
+    if not isinstance(segs, np.ndarray) or segs.dtype != _lib.SEGMENT_DTYPE or segs.ndim != 1:
+        raise ValueError("segs must be a 1-D numpy array of _lib.SEGMENT_DTYPE")
+    layer_begin = _render_begin(layer_begin, len(layers), "layer_begin")
+    seg_begin = _render_begin(seg_begin, len(segs), "seg_begin")
+    if len(layer_begin) != len(seg_begin):
+        raise ValueError("layer_begin and seg_begin must describe the same number of frames")
+    n_frames = len(layer_begin) - 1
+    n_masks = len(pool) if pool is not None else 0
+    if len(layers) and (np.any((layers["mask"] < 0) | (layers["mask"] >= n_masks))
+                        or np.any((layers["kind"] != _lib.LAYER_FILL) & (layers["kind"] != _lib.LAYER_OUTLINE))):
+        raise ValueError(f"a layer names a mask outside the pool of {n_masks} or an unknown kind")
+    if len(segs):
+        xy = np.stack([segs["x0"], segs["y0"], segs["x1"], segs["y1"]])
+        if np.any(np.abs(xy.astype(np.int64)) > _lib.RENDER_MAX_COORD) or \
+                np.any((segs["radius"] < 0) | (segs["radius"] > _lib.RENDER_MAX_RADIUS)):
+            raise ValueError(f"segment coordinates must lie within +-{_lib.RENDER_MAX_COORD} and radii in "
+                             f"[0, {_lib.RENDER_MAX_RADIUS}]")
+    if not torch.is_tensor(background) or background.dtype != torch.uint8 or background.dim() not in (3, 4) \
+            or background.shape[-1] != 3 or (background.dim() == 4 and background.shape[0] != n_frames):
+        raise ValueError(f"background must be a uint8 (H, W, 3) or ({n_frames}, H, W, 3) tensor")
+    H, W = int(background.shape[-3]), int(background.shape[-2])
+    if not (1 <= H <= _lib.RENDER_MAX_SIDE and 1 <= W <= _lib.RENDER_MAX_SIDE):
+        raise ValueError(f"a {H}x{W} frame is outside 1..{_lib.RENDER_MAX_SIDE} pixels a side")
+    if pool is not None and (pool.H, pool.W) != (H, W):
+        raise ValueError(f"mask pool is {pool.H}x{pool.W}, background is {H}x{W}")
+    if out is not None and (out.dtype != torch.uint8 or tuple(out.shape) != (n_frames, H, W, 3)
+                            or not out.is_contiguous()):
+        raise ValueError(f"out must be a contiguous uint8 ({n_frames}, {H}, {W}, 3) tensor")
+    lib = _lib.load()
+    _require_cuda(background, "background")
+    if pool is not None:
+        _require_cuda(pool.bits, "pool")
+    dev = background.device
+    background = background.contiguous()
+    # the four lists as one host block -> one H2D copy, every part 16-byte aligned
+    parts = [layers.view(np.uint8), segs.view(np.uint8), layer_begin.view(np.uint8), seg_begin.view(np.uint8)]
+    offs, total = [], 0
+    for p in parts:
+        offs.append(total)
+        total += (p.nbytes + 15) & ~15
+    host = np.zeros(max(total, 16), np.uint8)
+    for o, p in zip(offs, parts):
+        host[o:o + p.nbytes] = p
+    with torch.cuda.device(dev):
+        d = torch.from_numpy(host).to(dev)
+        base = d.data_ptr()
+        if out is None:
+            out = torch.empty(n_frames, H, W, 3, dtype=torch.uint8, device=dev)
+        else:
+            _require_cuda(out, "out")
+        stride = H * W * 3 if background.dim() == 4 else 0
+        _lib.check(lib.a3d_render(background.data_ptr(), stride, n_frames, H, W,
+                                  pool.bits.data_ptr() if pool is not None else None,
+                                  pool.bbox.data_ptr() if pool is not None else None, n_masks,
+                                  base + offs[0], base + offs[2], base + offs[1], base + offs[3],
+                                  out.data_ptr(), _stream_ptr()), "a3d_render")
+    return out

@@ -4,13 +4,15 @@ code); without it this tool runs on the synthetic detector stub (``synth.make_vi
 which emits the same ``Instances`` contract:
 
     python -m articulation3d_b200.tools.inference --frames 30 --tracks 4 --output out/ [--save-obj] [--save-textured-obj] \
-        [--save-masks]
+        [--save-masks] [--save-video [--fps 30]]
 
 ``--save-obj`` writes the geometry-only quads of ``io.write_obj``; ``--save-textured-obj`` the reference's export
 (``save_obj_model``, tools/inference.py:44-168, :282: object, rotated copies, axis markers, background, one
 300x300 texture each) through ``articulation3d_b200.export`` — with a flat grey image, the stub has no video.
 ``--save-masks`` adds every fitted frame's registered mask to ``<id>_tracks.json`` as COCO RLE (``segmentation`` of
-each ``angle_track`` entry).
+each ``angle_track`` entry).  ``--save-video`` writes ``<id>.mp4``: every frame drawn with the fitted result
+(``render.write_video``: registered masks, detection outlines, axes; reference tools/inference.py:253-278) on a flat
+grey background.
 """
 from __future__ import annotations
 
@@ -34,6 +36,8 @@ def main(argv=None):
     ap.add_argument("--save-obj", action="store_true")
     ap.add_argument("--save-textured-obj", action="store_true")
     ap.add_argument("--save-masks", action="store_true", help="registered masks (COCO RLE) in the tracks JSON")
+    ap.add_argument("--save-video", action="store_true", help="<output>/synthetic00_0_0.mp4 of the fitted result")
+    ap.add_argument("--fps", type=float, default=30)
     args = ap.parse_args(argv)
     random.seed(args.seed)                                   # tools/inference.py:172
     cfg = OptConfig()
@@ -56,6 +60,10 @@ def main(argv=None):
         from articulation3d_b200 import export
         for k in sorted({0, min(30, args.frames - 1), min(60, args.frames - 1), min(89, args.frames - 1)}):
             export.save_obj_model(args.output, opt_preds, k, image=None, cfg=cfg)                 # inference.py:282
+    if args.save_video:
+        from articulation3d_b200 import render
+        render.write_video(os.path.join(args.output, "synthetic00_0_0.mp4"), opt_preds, planes, fps=args.fps,
+                           cfg=cfg, device=args.device)
     print(f"{args.frames} frames, {len(planes['rot'])} rot + {len(planes['trans'])} trans tracks "
           f"in {dt * 1e3:.1f} ms -> {args.output}")
 

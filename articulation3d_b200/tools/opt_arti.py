@@ -1,7 +1,8 @@
 """Temporal optimisation of saved predictions — the B200 counterpart of the reference's
 ``tools/opt_arti.py`` for the stage in scope (the detector is not re-run):
 
-    python -m articulation3d_b200.tools.opt_arti --input instances_predictions.pth --output out/ [--save-obj] [--save-masks]
+    python -m articulation3d_b200.tools.opt_arti --input instances_predictions.pth --output out/ [--save-obj] [--save-masks] \
+        [--save-video [--fps 30] [--image-root DIR]]
     torchrun --nnodes 1 --nproc-per-node 8 -m articulation3d_b200.tools.opt_arti --input ... --output out/
 
 Reads the per-frame prediction records (RLE masks stay run-length encoded and are decoded on
@@ -9,7 +10,9 @@ the GPU), groups them by video, runs ``track_planes`` + ``optimize_planes('3dc')
 in lock-step, and writes per video ``<id>_predictions_opt.pth`` (records as
 tools/opt_arti.py:229-249), ``<id>_tracks.json`` (fitted axis + angle-per-frame track) and
 optionally ``<id>_frame<k>.obj``; ``--save-masks`` adds every fitted frame's registered mask to the tracks JSON
-as COCO RLE.  ``--override-depth`` first replaces every instance's plane offset by the one its record's
+as COCO RLE; ``--save-video`` writes ``<id>.mp4``, every frame drawn with the fitted result (``render.write_video``)
+over ``--image-root``/<record file_name> (flat grey without it; missing or wrongly sized images stop the tool before
+any device work).  ``--override-depth`` first replaces every instance's plane offset by the one its record's
 ``pred_depth`` implies (the reference's ``override_depth``), streamed through the GPU per rank.  ``--synthetic N``
 writes a synthetic input first (masks encoded on the tool's GPU; under torchrun rank 0 writes it on its own;
 ``--synthetic-depth`` adds a rendered ``pred_depth``).  The camera is the reference's 640x480 one scaled to the records' frame size
@@ -61,6 +64,32 @@ def frame_config(groups) -> OptConfig:
     return OptConfig() if (H, W) == (480, 640) else OptConfig.scaled(W, H)
 
 
+def _read_rgb(path: str):
+    import cv2
+    img = cv2.imread(path, cv2.IMREAD_COLOR) if os.path.isfile(path) else None
+    return None if img is None else cv2.cvtColor(img, cv2.COLOR_BGR2RGB)
+
+
+def check_images(root: str, order, cfg: OptConfig):
+    """Every record's ``root/<file_name>`` must be a readable image of the records' frame size; SystemExit with
+    the first offender otherwise.  Every rank checks every video, so a bad image stops all ranks alike."""
+    for _, recs in order:
+        for r in recs:
+            path = os.path.join(root, r["file_name"])
+            img = _read_rgb(path)
+            if img is None:
+                raise SystemExit(f"--image-root: cannot read {path}")
+            if img.shape[:2] != (cfg.height, cfg.width):
+                raise SystemExit(f"--image-root: {path} is {img.shape[1]}x{img.shape[0]}, the records' frames are "
+                                 f"{cfg.width}x{cfg.height}")
+
+
+def load_images(root: str, recs):
+    """(T, H, W, 3) uint8 RGB backgrounds of one video's records, in frame order."""
+    import numpy as np
+    return np.stack([_read_rgb(os.path.join(root, r["file_name"])) for r in recs])
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--input", required=True)
@@ -79,11 +108,17 @@ def main(argv=None):
     ap.add_argument("--override-depth", action="store_true", help="replace every instance's plane offset by the "
                     "mean over its mask of normal . XYZ of the record's pred_depth before tracking "
                     "(adapter.override_depth_records; tools/inference.py:220, tools/opt_arti.py:173-185)")
+    ap.add_argument("--save-video", action="store_true", help="<output>/<video id>.mp4 of the fitted result")
+    ap.add_argument("--fps", type=float, default=30)
+    ap.add_argument("--image-root", default=None, help="with --save-video: frame t is drawn over "
+                    "DIR/<record file_name> instead of a flat grey image")
     ap.add_argument("--tracks", type=int, default=4)
     ap.add_argument("--frames", type=int, default=60)
     args = ap.parse_args(argv)
     if args.synthetic_depth and not args.synthetic:
         ap.error("--synthetic-depth needs --synthetic N")
+    if args.image_root and not args.save_video:
+        ap.error("--image-root needs --save-video")
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world == 1:
@@ -155,6 +190,8 @@ def _run(args, rank: int, world: int, device: torch.device):
     order = list(adapter.group_by_video(adapter.load_predictions(args.input, mmap=world > 1)).items())
     cfg = frame_config(dict(order))
     mine = a3d_dist.shard_range(len(order), rank, world)
+    if args.image_root:
+        check_images(args.image_root, order, cfg)
     if args.override_depth:
         _override_depth(args, order, mine, rank, world, device)
     videos = [None] * len(order)                  # only this rank's block is converted and tracked
@@ -178,6 +215,11 @@ def _run(args, rank: int, world: int, device: torch.device):
         if args.save_obj:
             for k in (0, len(preds) // 3, 2 * len(preds) // 3, len(preds) - 1):
                 io.write_obj(os.path.join(args.output, f"{vid}_frame{k}.obj"), out, planes, k, cfg)
+        if args.save_video:
+            from articulation3d_b200 import render
+            images = load_images(args.image_root, recs) if args.image_root else None
+            render.write_video(os.path.join(args.output, f"{vid}.mp4"), out, planes, images=images, fps=args.fps,
+                               cfg=cfg, device=device, score_thresh=args.conf_threshold)
     if args.gt_json:
         if world == 1:
             after = [r for i, out in zip(mine, outs) for r in io.opt_preds_to_records(out, order[i][1])]

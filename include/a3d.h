@@ -292,6 +292,32 @@ int a3d_plane_offsets(const float* depth, const float* rays, int H, int W, const
                       const float* normals, int64_t n_inst, float* offset_out, int32_t* count_out,
                       void* stream);
 
+/* (f5) what a3d_render draws: a mask of the pool, filled or as its outline, blended with alpha rgba[3] */
+enum { A3D_LAYER_FILL = 0, A3D_LAYER_OUTLINE = 1 };
+typedef struct { int32_t mask; int32_t kind; uint8_t rgba[4]; } a3d_layer_t;                       /* 12 bytes */
+/* an opaque line segment of half-width `radius`; |coordinates| <= 2^14, 0 <= radius <= 256 */
+typedef struct { int32_t x0, y0, x1, y1; int32_t radius; uint8_t rgb[3], pad; } a3d_segment_t;    /* 24 bytes */
+#define A3D_RENDER_MAX_SIDE 16384
+
+/* (f5) the fitted result drawn into the clip's frames (reference tools/inference.py:253-278, there with
+ * detectron2's Visualizer): n_frames RGB frames out [n_frames][H][W][3] uint8, every byte defined as
+ *   1. the background pixel: background + f * bg_frame_stride (bytes; 0 = one H x W x 3 image for all frames);
+ *   2. frame f's layers layers[layer_begin[f] .. layer_begin[f+1]) in order: FILL covers the mask's set pixels,
+ *      OUTLINE its set pixels with at least one unset 4-neighbour (outside the frame = unset); a covered
+ *      channel o becomes (c * a + o * (255 - a) + 127) / 255 (uint32, floor);  a layer whose mask is outside
+ *      [0, n_masks) draws nothing;
+ *   3. frame f's segments segs[seg_begin[f] .. seg_begin[f+1]) in order, opaque: pixel q is on segment (p0, p1)
+ *      when its squared distance to the closed segment is <= radius^2, decided in int64 with d = p1 - p0,
+ *      t = (q - p0).d, L = d.d: t <= 0 -> |q - p0|^2, t >= L -> |q - p1|^2, else cross(q - p0, d)^2 <= r^2 L.
+ *   bits/bbox  the mask pool and its a3d_mask_meta boxes (bbox may be NULL: same output, no culling)
+ *   layers, layer_begin [n_frames + 1], segs, seg_begin [n_frames + 1]  DEVICE
+ * H, W <= A3D_RENDER_MAX_SIDE.  One CTA per (frame, band of rows): the band's background and output bytes
+ * are streamed once, the list entries whose box misses the band are culled first.                      */
+int a3d_render(const uint8_t* background, int64_t bg_frame_stride, int n_frames, int H, int W,
+               const uint32_t* bits, const int32_t* bbox, int64_t n_masks,
+               const a3d_layer_t* layers, const int64_t* layer_begin,
+               const a3d_segment_t* segs, const int64_t* seg_begin, uint8_t* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
