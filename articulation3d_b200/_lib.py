@@ -48,12 +48,18 @@ RENDER_MAX_SIDE = 16384      # A3D_RENDER_MAX_SIDE
 RENDER_MAX_COORD = 1 << 14   # |segment coordinate| limit of a3d_render
 RENDER_MAX_RADIUS = 256
 
+# a3d_plane_layer_t (a3d_plane_maps) as a numpy structured dtype, C layout
+PLANE_LAYER_DTYPE = np.dtype([("mask", "<i4"), ("normal", "<f4", (3,)), ("offset", "<f4"), ("rgb", "u1", (3,)),
+                              ("pad", "u1")])
+assert PLANE_LAYER_DTYPE.itemsize == 24
+
 # every symbol include/a3d.h declares
 EXPORTS = (
     "a3d_version", "a3d_last_error_string", "a3d_pitch_words", "a3d_project_max_tile",
     "a3d_pack_masks", "a3d_mask_meta", "a3d_project", "a3d_score", "a3d_pass", "a3d_emit_masks",
     "a3d_rle_to_bits", "a3d_plane_offsets", "a3d_plan_tiles", "a3d_host_quat_to_xform", "a3d_fetch_host_block", "a3d_upload_masks", "a3d_host_rle_counts",
     "a3d_rle_count_runs", "a3d_bits_to_rle", "a3d_host_rle_strings", "a3d_render",
+    "a3d_plane_maps",
 )
 
 _lib = None
@@ -118,6 +124,8 @@ def load():
     lib.a3d_plane_offsets.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp, vp]
     lib.a3d_render.restype = C.c_int
     lib.a3d_render.argtypes = [vp, i64, i32, i32, i32, vp, vp, i64, vp, vp, vp, vp, vp, vp]
+    lib.a3d_plane_maps.restype = C.c_int
+    lib.a3d_plane_maps.argtypes = [C.POINTER(Camera), i32, vp, vp, i64, vp, vp, vp, vp, vp, vp]
     _lib = lib
     return lib
 

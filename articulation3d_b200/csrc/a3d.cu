@@ -3352,3 +3352,161 @@ int a3d_render(const uint8_t* background, int64_t bg_frame_stride, int n_frames,
 }
 
 }  // extern "C"
+
+// ---------------------------------------------------------------------------
+// plane maps (a3d_plane_maps): per-pixel depth of the nearest planar mask and that mask's colour.
+// One CTA per (frame, band of rows).  The frame's layers whose box touches the band are culled into shared
+// memory kPlaneCap at a time, in list order; one warp takes one packed word of the band (32 pixels of a row),
+// one lane one pixel, and runs k_unproject's float64 ray/plane chain for every culled layer that has the pixel
+// set.  The band's running best (z, colour) lives in shared memory across the batches; the band's depth and
+// RGB bytes are written once at the end, contiguous and coalesced.  HBM traffic: the outputs and the mask
+// words inside the culled layers' boxes.
+// ---------------------------------------------------------------------------
+constexpr int kPlaneThreads = kRenderThreads;       // render_rank's block size
+constexpr int kPlaneCap = kPlaneThreads;            // layers culled per batch: one per thread
+constexpr int kPlaneBandPx = 4096;                  // target pixel slots (32 per packed word) of a band
+
+__global__ void __launch_bounds__(kPlaneThreads)
+k_plane_maps(const Cam cam, int f0, int band_rows, const uint32_t* __restrict__ bits, const int32_t* __restrict__ bbox,
+             int64_t n_masks, const a3d_plane_layer_t* __restrict__ layers, const int64_t* __restrict__ layer_begin,
+             uint32_t bg, float* __restrict__ depth_out, uint8_t* __restrict__ rgb_out) {
+    extern __shared__ float s_best[];               // [slots] running best z (+inf: none), then [slots] its rgb
+    __shared__ int4 s_lay[kPlaneCap];               // {mask, rgb, rows lo | hi << 16, words lo | hi << 16}
+    __shared__ float4 s_pl[kPlaneCap];              // {n0, n1, n2, offset}
+    __shared__ int s_warp[kPlaneThreads / 32];
+    const float INFf = __int_as_float(0x7f800000);
+    const int H = cam.H, W = cam.W, pitch = cam.pitch, nw = (W + 31) >> 5;
+    const int f = f0 + blockIdx.y;
+    const int r0 = blockIdx.x * band_rows, r1 = min(H, r0 + band_rows);
+    const int items = (r1 - r0) * nw;
+    float* s_z = s_best;
+    uint32_t* s_c = reinterpret_cast<uint32_t*>(s_best + band_rows * nw * 32);
+    for (int i = threadIdx.x; i < items * 32; i += kPlaneThreads) {
+        s_z[i] = INFf;
+        s_c[i] = bg;
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t le = layer_begin[f + 1];
+    for (int64_t li = layer_begin[f]; li < le; li += kPlaneCap) {
+        const int64_t k = li + threadIdx.x;
+        bool keep = false;
+        int4 e = make_int4(0, 0, 0, 0);
+        float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (k < le) {
+            const a3d_plane_layer_t L = layers[k];
+            if (L.mask >= 0 && L.mask < n_masks) {
+                int rmin = 0, rmax = H - 1, wmin = 0, wmax = nw - 1;
+                if (bbox) {
+                    const int4 b = ((const int4*)bbox)[L.mask];
+                    rmin = max(b.x, 0); rmax = min(b.y, H - 1); wmin = max(b.z, 0); wmax = min(b.w, nw - 1);
+                }
+                rmin = max(rmin, r0);
+                rmax = min(rmax, r1 - 1);
+                keep = rmin <= rmax && wmin <= wmax;
+                e = make_int4(L.mask, (int)(L.rgb[0] | (uint32_t)L.rgb[1] << 8 | (uint32_t)L.rgb[2] << 16),
+                              rmin | rmax << 16, wmin | wmax << 16);
+                p = make_float4(L.normal[0], L.normal[1], L.normal[2], L.offset);
+            }
+        }
+        int nl;
+        const int slot = render_rank(keep, s_warp, &nl);
+        if (keep) {
+            s_lay[slot] = e;
+            s_pl[slot] = p;
+        }
+        __syncthreads();
+        for (int it = warp; it < items; it += kPlaneThreads / 32) {
+            const int rr = it / nw, j = it - rr * nw, y = r0 + rr, x = 32 * j + lane;
+            if (x >= W) continue;
+            float best = s_z[32 * it + lane];
+            uint32_t col = s_c[32 * it + lane];
+            for (int q = 0; q < nl; ++q) {
+                const int4 L = s_lay[q];
+                if (y < (L.z & 0xffff) || y > (L.z >> 16) || j < (L.w & 0xffff) || j > (L.w >> 16)) continue;
+                const uint32_t word = bits[((int64_t)L.x * H + y) * pitch + j];
+                if (!((word >> lane) & 1u)) continue;
+                // the ray is recomputed per layer: nothing float64 stays live across the division's slow path
+                const double xd = (double)x, yd = (double)y;
+                double rx, ry, rz;
+                if (cam.sparse) {
+                    rx = __dadd_rn(__dmul_rn(cam.k[0], xd), cam.k[2]);
+                    ry = __dadd_rn(__dmul_rn(cam.k[4], yd), cam.k[5]);
+                    rz = 1.0;
+                } else {
+                    rx = __dadd_rn(__dadd_rn(__dmul_rn(cam.k[0], xd), __dmul_rn(cam.k[1], yd)), cam.k[2]);
+                    ry = __dadd_rn(__dadd_rn(__dmul_rn(cam.k[3], xd), __dmul_rn(cam.k[4], yd)), cam.k[5]);
+                    rz = __dadd_rn(__dadd_rn(__dmul_rn(cam.k[6], xd), __dmul_rn(cam.k[7], yd)), cam.k[8]);
+                }
+                const float4 P = s_pl[q];
+                const double dot = __dadd_rn(__dadd_rn(__dmul_rn((double)P.x, rx), __dmul_rn((double)P.y, ry)),
+                                             __dmul_rn((double)P.z, rz));
+                const float z = __double2float_rn(__dmul_rn(__ddiv_rn((double)P.w, dot), rz));
+                if (z > 0.f && z < best) {         // best <= +inf: a finite z only; NaN fails both; ties keep the first
+                    best = z;
+                    col = (uint32_t)L.y;
+                }
+            }
+            s_z[32 * it + lane] = best;
+            s_c[32 * it + lane] = col;
+        }
+        __syncthreads();
+    }
+    __syncthreads();
+    for (int rr = 0; rr < r1 - r0; ++rr) {          // row by row: no division by W per output element
+        const int64_t row = (int64_t)f * H + r0 + rr;
+        if (depth_out) {
+            const float* zr = s_z + 32 * rr * nw;
+            float* o = depth_out + row * W;
+            for (int x = threadIdx.x; x < W; x += kPlaneThreads) {
+                const float z = zr[x];
+                o[x] = z < INFf ? z : 0.f;
+            }
+        }
+        if (rgb_out) {
+            const uint32_t* cr = s_c + 32 * rr * nw;
+            uint8_t* o = rgb_out + row * W * 3;
+            for (int i = threadIdx.x; i < 3 * W; i += kPlaneThreads) {
+                const int px = (int)((unsigned)i / 3u);
+                o[i] = (uint8_t)(cr[px] >> (8 * (i - 3 * px)));
+            }
+        }
+    }
+}
+
+extern "C" {
+
+int a3d_plane_maps(const a3d_camera_t* cam, int n_frames, const uint32_t* bits, const int32_t* bbox, int64_t n_masks,
+                   const a3d_plane_layer_t* layers, const int64_t* layer_begin, const uint8_t bg_rgb[3],
+                   float* depth_out, uint8_t* rgb_out, void* stream) {
+    if (!cam) return fail(A3D_EINVAL, "a3d_plane_maps: null camera");
+    const int H = cam->H, W = cam->W;
+    if (n_frames < 0 || H <= 0 || W <= 0 || n_masks < 0)
+        return fail(A3D_EINVAL, "a3d_plane_maps: bad shape n_frames=%d %dx%d n_masks=%lld", n_frames, H, W,
+                    (long long)n_masks);
+    if (H > A3D_RENDER_MAX_SIDE || W > A3D_RENDER_MAX_SIDE)
+        return fail(A3D_ELIMIT, "a3d_plane_maps: %dx%d frame exceeds %d pixels a side", H, W, A3D_RENDER_MAX_SIDE);
+    if (n_frames == 0 || (!depth_out && !rgb_out)) return A3D_OK;
+    if (!layer_begin || (n_masks > 0 && !bits) || (rgb_out && !bg_rgb))
+        return fail(A3D_EINVAL, "a3d_plane_maps: null pointer");
+    Cam c;
+    memcpy(c.k, cam->kinv, sizeof(c.k));
+    c.f = cam->f; c.cx = cam->cx; c.cy = cam->cy;
+    c.H = H; c.W = W; c.pitch = pitch_words(W);
+    c.sparse = (c.k[1] == 0.0 && c.k[3] == 0.0 && c.k[6] == 0.0 && c.k[7] == 0.0 && c.k[8] == 1.0);
+    const uint32_t bg = rgb_out ? (bg_rgb[0] | (uint32_t)bg_rgb[1] << 8 | (uint32_t)bg_rgb[2] << 16) : 0u;
+    const int row_slots = 32 * ((W + 31) >> 5);
+    int band_rows = kPlaneBandPx / row_slots;
+    band_rows = band_rows < 1 ? 1 : (band_rows > H ? H : band_rows);
+    const int smem = band_rows * row_slots * 8;
+    A3D_CUDA_TRY(cudaFuncSetAttribute(k_plane_maps, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    const unsigned bands = (unsigned)((H + band_rows - 1) / band_rows);
+    for (int f0 = 0; f0 < n_frames; f0 += 65535) {
+        const unsigned nf = (unsigned)(n_frames - f0 < 65535 ? n_frames - f0 : 65535);
+        k_plane_maps<<<dim3(bands, nf), kPlaneThreads, smem, (cudaStream_t)stream>>>(
+            c, f0, band_rows, bits, bbox, n_masks, layers, layer_begin, bg, depth_out, rgb_out);
+        A3D_CUDA_TRY(cudaGetLastError());
+    }
+    return A3D_OK;
+}
+
+}  // extern "C"

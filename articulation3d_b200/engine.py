@@ -843,3 +843,69 @@ def render(pool: MaskPool | None, layers: np.ndarray, layer_begin, segs: np.ndar
                                   base + offs[0], base + offs[2], base + offs[1], base + offs[3],
                                   out.data_ptr(), _stream_ptr()), "a3d_render")
     return out
+
+
+def plane_maps(pool: MaskPool | None, layers: np.ndarray, layer_begin, cfg: OptConfig, bg_rgb=(0, 0, 0),
+               depth_out: torch.Tensor | None = None, rgb_out: torch.Tensor | None = None, device=None):
+    """Per-frame depth and colour maps of planar masks on the device (``a3d_plane_maps``).
+
+    ``layers`` (``_lib.PLANE_LAYER_DTYPE``) is a host array; frame f draws ``layers[layer_begin[f]:layer_begin[f+1]]``:
+    every layer covers the set pixels of its ``pool`` mask where the pixel's ray (``cfg.K_inv()``) meets the layer's
+    plane ``normal . X = offset`` in front of the camera, and the nearest covering layer wins (the earlier one on a
+    tie).  Returns ``(depth, rgb)``: (n_frames, H, W) fp32 z (0 where nothing covers the pixel) and
+    (n_frames, H, W, 3) uint8 (``bg_rgb`` where nothing does), on the pool's device (``depth_out`` / ``rgb_out`` if
+    given; ``device`` when there is no pool).  Everything from outside is checked before the launch: ValueError
+    for bad lists, limits or shapes."""
+    if not isinstance(layers, np.ndarray) or layers.dtype != _lib.PLANE_LAYER_DTYPE or layers.ndim != 1:
+        raise ValueError("layers must be a 1-D numpy array of _lib.PLANE_LAYER_DTYPE")
+    layer_begin = _render_begin(layer_begin, len(layers), "layer_begin")
+    n_frames = len(layer_begin) - 1
+    n_masks = len(pool) if pool is not None else 0
+    if len(layers) and np.any((layers["mask"] < 0) | (layers["mask"] >= n_masks)):
+        raise ValueError(f"a layer names a mask outside the pool of {n_masks}")
+    bg = np.asarray(bg_rgb)
+    if bg.shape != (3,) or bg.dtype.kind not in "iu" or np.any((bg < 0) | (bg > 255)):
+        raise ValueError("bg_rgb must be three integers in [0, 255]")
+    H, W = int(cfg.height), int(cfg.width)
+    if not (1 <= H <= _lib.RENDER_MAX_SIDE and 1 <= W <= _lib.RENDER_MAX_SIDE):
+        raise ValueError(f"a {H}x{W} frame is outside 1..{_lib.RENDER_MAX_SIDE} pixels a side")
+    if pool is not None and (pool.H, pool.W) != (H, W):
+        raise ValueError(f"mask pool is {pool.H}x{pool.W}, camera is {H}x{W}")
+    if depth_out is not None and (depth_out.dtype != torch.float32 or tuple(depth_out.shape) != (n_frames, H, W)
+                                  or not depth_out.is_contiguous()):
+        raise ValueError(f"depth_out must be a contiguous fp32 ({n_frames}, {H}, {W}) tensor")
+    if rgb_out is not None and (rgb_out.dtype != torch.uint8 or tuple(rgb_out.shape) != (n_frames, H, W, 3)
+                                or not rgb_out.is_contiguous()):
+        raise ValueError(f"rgb_out must be a contiguous uint8 ({n_frames}, {H}, {W}, 3) tensor")
+    lib = _lib.load()
+    if pool is not None:
+        _require_cuda(pool.bits, "pool")
+        dev = pool.bits.device
+    else:
+        dev = torch.device(device if device is not None else "cuda")
+        if dev.type != "cuda" or not torch.cuda.is_available():
+            raise _lib.A3DError("plane_maps needs a CUDA device (the hot path has no CPU fallback)")
+    for t, name in ((depth_out, "depth_out"), (rgb_out, "rgb_out")):
+        if t is not None:
+            _require_cuda(t, name)
+            if t.device != dev:
+                raise ValueError(f"{name} is on {t.device}, the masks on {dev}")
+    # the two lists as one host block -> one H2D copy, both parts 16-byte aligned
+    lay, beg = layers.view(np.uint8), layer_begin.view(np.uint8)
+    off = (lay.nbytes + 15) & ~15
+    host = np.zeros(max(off + beg.nbytes, 16), np.uint8)
+    host[:lay.nbytes] = lay
+    host[off:off + beg.nbytes] = beg
+    bg_c = (C.c_uint8 * 3)(*(int(v) for v in bg))
+    with torch.cuda.device(dev):
+        d = torch.from_numpy(host).to(dev)
+        if depth_out is None:
+            depth_out = torch.empty(n_frames, H, W, dtype=torch.float32, device=dev)
+        if rgb_out is None:
+            rgb_out = torch.empty(n_frames, H, W, 3, dtype=torch.uint8, device=dev)
+        cam = camera_struct(cfg)                  # cfg.K_inv() as it is now (no cache keyed on f, W, H)
+        _lib.check(lib.a3d_plane_maps(C.byref(cam), n_frames, pool.bits.data_ptr() if pool is not None else None,
+                                      pool.bbox.data_ptr() if pool is not None else None, n_masks,
+                                      d.data_ptr(), d.data_ptr() + off, bg_c, depth_out.data_ptr(),
+                                      rgb_out.data_ptr(), _stream_ptr()), "a3d_plane_maps")
+    return depth_out, rgb_out

@@ -252,3 +252,38 @@ def transform_normals(normal: torch.Tensor, R: np.ndarray) -> torch.Tensor:
     m = torch.from_numpy(np.ascontiguousarray(R))
     n = normal.reshape(1, 1, 3).expand(len(m), -1, -1)
     return n.bmm(m.transpose(1, 2).inverse())[:, 0]
+
+
+def registered_planes(normal: torch.Tensor, offset, xform_rows: np.ndarray, mode: int, pivot, cand,
+                      normals: torch.Tensor | None = None) -> np.ndarray:
+    """Planes of the source mask moved by candidates ``cand`` of a job: (len(cand), 4) fp32 rows [n', d'] with
+    n' . p' = d' for every point p' = p R + t of the moved plane n . p = offset (camera frame of get_pcd).
+
+    ``xform_rows`` (A, 12) are the job's candidate rows (R row-major, t).  n' = n (R^T)^-1 is
+    ``transform_normals`` (the fp32 value ``reg_normals`` is built from; ``normals`` may pass it in when already
+    computed for all A rows); R = I for ``MODE_TRANSLATE`` (n' = n); for ``MODE_SEQ`` t = a - a R with a the fp32
+    ``pivot``, in float64.  d' = fp32 of the float64 d + n'.t, exact for any invertible R:
+    n . p = d  <=>  n' . p' = d + n' . t."""
+    from . import _lib
+    rows = np.asarray(xform_rows, dtype=np.float32).reshape(-1, 12)
+    cand = np.asarray(cand, dtype=np.int64).reshape(-1)
+    R = rows[:, :9].reshape(-1, 3, 3)
+    if mode == _lib.MODE_TRANSLATE:
+        n_sel = np.broadcast_to(normal.detach().cpu().numpy().astype(np.float32).reshape(1, 3), (len(cand), 3))
+    else:
+        if normals is None:
+            normals = transform_normals(normal, R)
+        n_sel = normals.numpy()[cand]
+    Rs = R[cand].astype(np.float64)
+    if mode == _lib.MODE_SEQ:
+        a = np.asarray(pivot, dtype=np.float32).astype(np.float64)
+        t = a[None, :] - ((a[0] * Rs[:, 0, :] + a[1] * Rs[:, 1, :]) + a[2] * Rs[:, 2, :])
+    else:
+        t = rows[cand, 9:].astype(np.float64)
+    n64 = n_sel.astype(np.float64)
+    with np.errstate(all="ignore"):
+        d = np.float64(np.float32(float(offset))) + ((n64[:, 0] * t[:, 0] + n64[:, 1] * t[:, 1]) + n64[:, 2] * t[:, 2])
+    out = np.empty((len(cand), 4), dtype=np.float32)
+    out[:, :3] = n_sel
+    out[:, 3] = d.astype(np.float32)
+    return out

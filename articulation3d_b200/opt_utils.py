@@ -421,6 +421,7 @@ def _tracks_gen(preds, planes, cfg: OptConfig, translation: bool, rng, pool_of, 
         frames = list(plane['ids'].keys())
         stats.units_visited += len(fgrid) * len(frames)
         plane['reg_masks'] = RegMasks(frames, res.masks, H, W)
+        normal_trans = None
         if fmode == _lib.MODE_COMPOSED:
             normal_trans = geometry.transform_normals(geo.normal, R_all[k])
             sel = normal_trans[torch.from_numpy(res.best_cand.astype(np.int64))]
@@ -436,6 +437,9 @@ def _tracks_gen(preds, planes, cfg: OptConfig, translation: bool, rng, pool_of, 
             'frames': frames, 'center_frame': select_idx, 'rsq': rsqs, 'clusters': clusters,
             'angle_id': res.best_cand.copy(), 'angle': angles_f[:, 0].numpy()[res.best_cand],
             'inter': res.best_inter.copy(), 'union': res.best_union.copy(), 'iou': res.best_iou.copy(),
+            # the plane of every fitted frame's registered mask, [n', d'] in get_pcd's camera frame
+            'reg_plane': geometry.registered_planes(geo.normal, geo.offset, xf_all[k], fmode, geo.pivot,
+                                                    res.best_cand, normals=normal_trans),
         }
 
 

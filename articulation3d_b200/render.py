@@ -18,13 +18,21 @@ Tracks are numbered as ``io.tracks_summary`` lists them (``trans``, then ``rot``
 ``draw_lists`` builds the per-frame draw lists on the host; ``render_clip`` composites them on the device with
 ``engine.render`` straight from the packed registered masks (no dense mask is made); ``write_video`` renders
 bounded chunks of frames and encodes one chunk on the host while the next renders.
+
+The 3-D half of the result (row f6): ``plane_lists`` puts every fitted track's registered mask on its registered
+plane (``plane['fit']['reg_plane']``) and every other detection above the threshold on its own plane;
+``plane_maps`` turns them into per-frame depth and surface-normal maps on the device (``engine.plane_maps``: the
+nearest plane wins each pixel), and ``write_plane_maps`` writes them as 16-bit millimetre PNGs and a normal-map mp4
+through the same chunked pipeline as ``write_video``.
 """
 from __future__ import annotations
 
+import os
 from dataclasses import dataclass
 
 import numpy as np
 import torch
+import torch.nn.functional as F
 
 from . import _lib, engine
 from .axis import angle_offset_to_axis_rows
@@ -190,6 +198,38 @@ def render_clip(opt_preds, planes, images=None, cfg: OptConfig | None = None, de
         return _render_range(pool, lists, bg, 0, len(opt_preds), device)
 
 
+def _stream_chunks(T: int, per: int, parts, produce, consume, device):
+    """Bounded-chunk device -> host pipeline: ``produce(a, b)`` returns device tensors for frames [a, b) shaped
+    like ``parts`` ((frame shape, dtype) each); they are copied into one of two sets of pinned host buffers, and
+    ``consume(a, host tensors)`` runs on the host for a chunk while the device produces and copies the next."""
+    with torch.cuda.device(device):
+        pinned = [[torch.empty((per,) + tuple(shape), dtype=dt).pin_memory() for shape, dt in parts]
+                  for _ in range(min(2, -(-T // per)))]
+        pending = None
+        for c, a in enumerate(range(0, T, per)):
+            b = min(T, a + per)
+            hosts = [buf[:b - a] for buf in pinned[c % 2]]
+            for host, dev in zip(hosts, produce(a, b)):
+                host.copy_(dev, non_blocking=True)
+            done = torch.cuda.Event()
+            done.record()
+            if pending is not None:
+                pending[0].synchronize()
+                consume(*pending[1:])              # the previous chunk, while this one is produced and copied
+            pending = (done, a, hosts)
+        if pending is not None:
+            pending[0].synchronize()
+            consume(*pending[1:])
+
+
+def _video_writer(path: str, fps: float, W: int, H: int):
+    import cv2
+    writer = cv2.VideoWriter(path, cv2.VideoWriter_fourcc(*"mp4v"), float(fps), (W, H))
+    if not writer.isOpened():
+        raise RuntimeError(f"cv2.VideoWriter cannot open {path}")
+    return writer
+
+
 def write_video(path: str, opt_preds, planes, images=None, fps: float = 30, cfg: OptConfig | None = None,
                 device=None, score_thresh: float = 0.7, chunk_bytes: int = 64 << 20) -> str:
     """``render_clip`` written as an mp4 (``cv2.VideoWriter``, ``mp4v``).  Frames are rendered in chunks of at most
@@ -204,31 +244,138 @@ def write_video(path: str, opt_preds, planes, images=None, fps: float = 30, cfg:
     pool = mask_pool(opt_preds, lists, cfg, device)
     bg = _background(images, T, H, W, device)
     per = max(1, min(T, chunk_bytes // (H * W * 3)))
-    writer = cv2.VideoWriter(path, cv2.VideoWriter_fourcc(*"mp4v"), float(fps), (W, H))
-    if not writer.isOpened():
-        raise RuntimeError(f"cv2.VideoWriter cannot open {path}")
+    writer = _video_writer(path, fps, W, H)
 
-    def encode(host, done):
-        done.synchronize()
-        for frame in host.numpy():
+    def encode(a, hosts):
+        for frame in hosts[0].numpy():
             writer.write(cv2.cvtColor(frame, cv2.COLOR_RGB2BGR))
 
     try:
-        with torch.cuda.device(device):
-            pinned = [torch.empty((per, H, W, 3), dtype=torch.uint8).pin_memory() for _ in range(min(2, -(-T // per)))]
-            pending = None
-            for c, a in enumerate(range(0, T, per)):
-                b = min(T, a + per)
-                frames = _render_range(pool, lists, bg, a, b, device)
-                host = pinned[c % 2][:b - a]
-                host.copy_(frames, non_blocking=True)
-                done = torch.cuda.Event()
-                done.record()
-                if pending is not None:
-                    encode(*pending)               # the previous chunk, while this one renders and copies
-                pending = (host, done)
-            if pending is not None:
-                encode(*pending)
+        _stream_chunks(T, per, [((H, W, 3), torch.uint8)],
+                       lambda a, b: [_render_range(pool, lists, bg, a, b, device)], encode, device)
     finally:
         writer.release()
     return path
+
+
+# ---------------------------------------------------------------------------
+# depth and surface-normal maps of the fitted planes (row f6)
+# ---------------------------------------------------------------------------
+@dataclass
+class PlaneLists:
+    """Per-frame plane layers of a clip, indexing the same pool as ``DrawLists`` (``mask_pool`` builds it): the
+    registered masks of every fitted track in track order, then every detection mask in (frame, box) order."""
+    layers: np.ndarray           # _lib.PLANE_LAYER_DTYPE
+    layer_begin: np.ndarray      # (T + 1,) int64
+    fitted: list                 # plane dicts of the fitted tracks, in pool order
+    n_reg: int                   # registered masks at the front of the pool
+
+
+def normal_colours(normals) -> np.ndarray:
+    """(n, 3) uint8 colours of fp32 unit normals: clamp(floor(127.5 (1 - n_i) + 0.5), 0, 255) in float64 (a NaN
+    component gives 0).  A visible plane has n . ray > 0, so this colours the camera-facing normal -n."""
+    n = np.asarray(normals, dtype=np.float32).astype(np.float64).reshape(-1, 3)
+    c = np.floor(127.5 * (1.0 - n) + 0.5)
+    return np.clip(np.nan_to_num(c, nan=0.0), 0, 255).astype(np.uint8)
+
+
+def detection_planes(pred_planes) -> tuple[np.ndarray, np.ndarray]:
+    """(normal (n, 3), offset (n,)) fp32 of detector plane rows, as ``geometry.source_geometry`` converts them:
+    [a, b, c] -> [a, -c, b], normal = p / |p|, offset = |p|."""
+    plane = torch.as_tensor(pred_planes).detach().cpu().to(torch.float32).clone().reshape(-1, 3)
+    plane[:, [1, 2]] = plane[:, [2, 1]]
+    plane[:, 1] = -plane[:, 1]
+    return F.normalize(plane, p=2).numpy(), torch.norm(plane, p=2, dim=1).numpy()
+
+
+def plane_lists(opt_preds, planes, cfg: OptConfig | None = None, score_thresh: float = 0.7) -> PlaneLists:
+    """Plane layers of every frame of a clip (host only).  Per frame: every fitted track's registered mask on its
+    ``fit['reg_plane']`` row, then every detection with score >= ``score_thresh`` whose box is not a fitted track's
+    at that frame, on its own plane (``detection_planes``); each coloured by its normal (``normal_colours``)."""
+    T = len(opt_preds)
+    fitted = [pl for _, pl in _tracks(planes) if pl.get("has_rot", False)]
+    rows = [[] for _ in range(T)]
+    owned = set()
+    base = 0
+    for pl in fitted:
+        reg = np.asarray(pl["fit"]["reg_plane"], dtype=np.float32).reshape(-1, 4)
+        if len(reg) != len(pl["ids"]):
+            raise ValueError(f"fit['reg_plane'] has {len(reg)} rows for {len(pl['ids'])} fitted frames")
+        cols = normal_colours(reg[:, :3])
+        for i, (f, b) in enumerate(pl["ids"].items()):
+            rows[f].append((base + i, reg[i, :3], reg[i, 3], cols[i], 0))
+            owned.add((int(f), int(b)))
+        base += len(pl["ids"])
+    n_reg = base
+    for f, p in enumerate(opt_preds):
+        scores = np.asarray(p.scores, dtype=np.float64).reshape(-1)
+        keep = [int(b) for b in np.flatnonzero(scores >= score_thresh) if (f, int(b)) not in owned]
+        if keep:
+            normal, offset = detection_planes(torch.as_tensor(p.pred_planes)[keep])
+            cols = normal_colours(normal)
+            for i, b in enumerate(keep):
+                rows[f].append((base + b, normal[i], offset[i], cols[i], 0))
+        base += len(scores)
+    layers, begin = _flatten(rows, _lib.PLANE_LAYER_DTYPE)
+    return PlaneLists(layers, begin, fitted, n_reg)
+
+
+def _plane_range(pool, lists: PlaneLists, cfg: OptConfig, a: int, b: int, device, bg_rgb=(0, 0, 0)):
+    lb = lists.layer_begin
+    return engine.plane_maps(pool, lists.layers[lb[a]:lb[b]], lb[a:b + 1] - lb[a], cfg, bg_rgb, device=device)
+
+
+def plane_maps(opt_preds, planes, cfg: OptConfig | None = None, device=None, score_thresh: float = 0.7,
+               bg_rgb=(0, 0, 0)):
+    """(depth (T, H, W) fp32, rgb (T, H, W, 3) uint8) CUDA tensors of the clip's planes: every pixel's z of the
+    nearest plane layer covering it (0 where none does) and that layer's normal colour (``bg_rgb`` where none)."""
+    cfg = cfg or OptConfig()
+    device = _device(device, planes)
+    lists = plane_lists(opt_preds, planes, cfg, score_thresh)
+    pool = mask_pool(opt_preds, lists, cfg, device)
+    with torch.cuda.device(device):
+        return _plane_range(pool, lists, cfg, 0, len(opt_preds), device)
+
+
+def depth_millimetres(depth: torch.Tensor) -> torch.Tensor:
+    """uint16 millimetres of fp32 metres as int16 bits (torch has no uint16 arithmetic):
+    (z * 1000).round().clamp(0, 65535) in fp32 on the tensor's device; 0 = no plane."""
+    mm = (depth * 1000.0).round_().clamp_(0, 65535).to(torch.int32)
+    return mm.view(torch.int16).reshape(depth.shape + (2,))[..., 0].contiguous()     # low half, little endian
+
+
+def write_plane_maps(out_dir: str, video_id: str, opt_preds, planes, fps: float = 30, cfg: OptConfig | None = None,
+                     device=None, score_thresh: float = 0.7, chunk_bytes: int = 64 << 20) -> tuple[str, str]:
+    """``plane_maps`` written as ``<out_dir>/<video_id>_depth/<k:05d>.png`` (uint16 millimetres, k = the frame's
+    position in the clip) and ``<out_dir>/<video_id>_normals.mp4`` (cv2 ``mp4v``, black where no plane is).
+    Chunks of at most ``chunk_bytes`` of depth + RGB go through pinned buffers as in ``write_video``.  Returns the
+    directory and the video path."""
+    import cv2
+    cfg = cfg or OptConfig()
+    H, W = cfg.height, cfg.width
+    T = len(opt_preds)
+    device = _device(device, planes)
+    lists = plane_lists(opt_preds, planes, cfg, score_thresh)
+    pool = mask_pool(opt_preds, lists, cfg, device)
+    depth_dir = os.path.join(out_dir, f"{video_id}_depth")
+    os.makedirs(depth_dir, exist_ok=True)
+    path = os.path.join(out_dir, f"{video_id}_normals.mp4")
+    per = max(1, min(T, chunk_bytes // (H * W * 5)))
+    writer = _video_writer(path, fps, W, H)
+
+    def produce(a, b):
+        depth, rgb = _plane_range(pool, lists, cfg, a, b, device)
+        return [depth_millimetres(depth), rgb]
+
+    def encode(a, hosts):
+        mm, rgb = hosts
+        for i, (d, frame) in enumerate(zip(mm.numpy(), rgb.numpy())):
+            if not cv2.imwrite(os.path.join(depth_dir, f"{a + i:05d}.png"), d.view(np.uint16)):
+                raise RuntimeError(f"cv2.imwrite cannot write {depth_dir}/{a + i:05d}.png")
+            writer.write(cv2.cvtColor(frame, cv2.COLOR_RGB2BGR))
+
+    try:
+        _stream_chunks(T, per, [((H, W), torch.int16), ((H, W, 3), torch.uint8)], produce, encode, device)
+    finally:
+        writer.release()
+    return depth_dir, path

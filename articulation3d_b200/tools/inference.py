@@ -4,7 +4,7 @@ code); without it this tool runs on the synthetic detector stub (``synth.make_vi
 which emits the same ``Instances`` contract:
 
     python -m articulation3d_b200.tools.inference --frames 30 --tracks 4 --output out/ [--save-obj] [--save-textured-obj] \
-        [--save-masks] [--save-video [--fps 30]]
+        [--save-masks] [--save-video [--fps 30]] [--save-depth]
 
 ``--save-obj`` writes the geometry-only quads of ``io.write_obj``; ``--save-textured-obj`` the reference's export
 (``save_obj_model``, tools/inference.py:44-168, :282: object, rotated copies, axis markers, background, one
@@ -12,7 +12,9 @@ which emits the same ``Instances`` contract:
 ``--save-masks`` adds every fitted frame's registered mask to ``<id>_tracks.json`` as COCO RLE (``segmentation`` of
 each ``angle_track`` entry).  ``--save-video`` writes ``<id>.mp4``: every frame drawn with the fitted result
 (``render.write_video``: registered masks, detection outlines, axes; reference tools/inference.py:253-278) on a flat
-grey background.
+grey background.  ``--save-depth`` writes the fitted planes' per-frame depth as ``<id>_depth/<k:05d>.png`` (uint16
+millimetres, 0 = no plane) and their surface normals as ``<id>_normals.mp4`` (``render.write_plane_maps``; reference
+tools/inference.py:231-243 shows the normal map).
 """
 from __future__ import annotations
 
@@ -38,6 +40,8 @@ def main(argv=None):
     ap.add_argument("--save-masks", action="store_true", help="registered masks (COCO RLE) in the tracks JSON")
     ap.add_argument("--save-video", action="store_true", help="<output>/synthetic00_0_0.mp4 of the fitted result")
     ap.add_argument("--fps", type=float, default=30)
+    ap.add_argument("--save-depth", action="store_true", help="<output>/synthetic00_0_0_depth/<k>.png (uint16 mm) and "
+                    "synthetic00_0_0_normals.mp4 of the fitted planes")
     args = ap.parse_args(argv)
     random.seed(args.seed)                                   # tools/inference.py:172
     cfg = OptConfig()
@@ -64,6 +68,10 @@ def main(argv=None):
         from articulation3d_b200 import render
         render.write_video(os.path.join(args.output, "synthetic00_0_0.mp4"), opt_preds, planes, fps=args.fps,
                            cfg=cfg, device=args.device)
+    if args.save_depth:
+        from articulation3d_b200 import render
+        render.write_plane_maps(args.output, "synthetic00_0_0", opt_preds, planes, fps=args.fps, cfg=cfg,
+                                device=args.device)
     print(f"{args.frames} frames, {len(planes['rot'])} rot + {len(planes['trans'])} trans tracks "
           f"in {dt * 1e3:.1f} ms -> {args.output}")
 

@@ -2,7 +2,7 @@
 ``tools/opt_arti.py`` for the stage in scope (the detector is not re-run):
 
     python -m articulation3d_b200.tools.opt_arti --input instances_predictions.pth --output out/ [--save-obj] [--save-masks] \
-        [--save-video [--fps 30] [--image-root DIR]]
+        [--save-video [--fps 30] [--image-root DIR]] [--save-depth]
     torchrun --nnodes 1 --nproc-per-node 8 -m articulation3d_b200.tools.opt_arti --input ... --output out/
 
 Reads the per-frame prediction records (RLE masks stay run-length encoded and are decoded on
@@ -12,7 +12,9 @@ tools/opt_arti.py:229-249), ``<id>_tracks.json`` (fitted axis + angle-per-frame 
 optionally ``<id>_frame<k>.obj``; ``--save-masks`` adds every fitted frame's registered mask to the tracks JSON
 as COCO RLE; ``--save-video`` writes ``<id>.mp4``, every frame drawn with the fitted result (``render.write_video``)
 over ``--image-root``/<record file_name> (flat grey without it; missing or wrongly sized images stop the tool before
-any device work).  ``--override-depth`` first replaces every instance's plane offset by the one its record's
+any device work); ``--save-depth`` writes ``<id>_depth/<k:05d>.png`` (per-frame depth of the fitted planes, uint16
+millimetres, 0 = no plane) and ``<id>_normals.mp4`` (their surface normals; ``render.write_plane_maps``, detections
+gated by ``--conf-threshold``).  ``--override-depth`` first replaces every instance's plane offset by the one its record's
 ``pred_depth`` implies (the reference's ``override_depth``), streamed through the GPU per rank.  ``--synthetic N``
 writes a synthetic input first (masks encoded on the tool's GPU; under torchrun rank 0 writes it on its own;
 ``--synthetic-depth`` adds a rendered ``pred_depth``).  The camera is the reference's 640x480 one scaled to the records' frame size
@@ -112,6 +114,8 @@ def main(argv=None):
     ap.add_argument("--fps", type=float, default=30)
     ap.add_argument("--image-root", default=None, help="with --save-video: frame t is drawn over "
                     "DIR/<record file_name> instead of a flat grey image")
+    ap.add_argument("--save-depth", action="store_true", help="<output>/<video id>_depth/<k>.png (uint16 mm) and "
+                    "<video id>_normals.mp4 of the fitted planes")
     ap.add_argument("--tracks", type=int, default=4)
     ap.add_argument("--frames", type=int, default=60)
     args = ap.parse_args(argv)
@@ -220,6 +224,10 @@ def _run(args, rank: int, world: int, device: torch.device):
             images = load_images(args.image_root, recs) if args.image_root else None
             render.write_video(os.path.join(args.output, f"{vid}.mp4"), out, planes, images=images, fps=args.fps,
                                cfg=cfg, device=device, score_thresh=args.conf_threshold)
+        if args.save_depth:
+            from articulation3d_b200 import render
+            render.write_plane_maps(args.output, vid, out, planes, fps=args.fps, cfg=cfg, device=device,
+                                    score_thresh=args.conf_threshold)
     if args.gt_json:
         if world == 1:
             after = [r for i, out in zip(mine, outs) for r in io.opt_preds_to_records(out, order[i][1])]

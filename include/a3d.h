@@ -318,6 +318,30 @@ int a3d_render(const uint8_t* background, int64_t bg_frame_stride, int n_frames,
                const a3d_layer_t* layers, const int64_t* layer_begin,
                const a3d_segment_t* segs, const int64_t* seg_begin, uint8_t* out, void* stream);
 
+/* (f6) a mask of the pool lying on the plane n . X = offset (camera frame of get_pcd), drawn in colour rgb */
+typedef struct { int32_t mask; float normal[3]; float offset; uint8_t rgb[3], pad; } a3d_plane_layer_t;   /* 24 bytes */
+
+/* (f6) per-frame depth and colour (e.g. surface-normal) maps of planar masks (reference tools/inference.py:231-243
+ * shows the planes as a normal map).  For pixel (x, y) of frame f and every layer of
+ * layers[layer_begin[f] .. layer_begin[f+1]) whose mask has the pixel set, in float64 with every product and sum
+ * rounded separately, left to right (k_unproject's chain):
+ *     ray = kinv [x, y, 1]   (rx = (k0 x + k1 y) + k2, ry = (k3 x + k4 y) + k5, rz = (k6 x + k7 y) + k8;
+ *                             with k1 = k3 = k6 = k7 = 0, k8 = 1: rx = k0 x + k2, ry = k4 y + k5, rz = 1)
+ *     dot = (n0 rx + n1 ry) + n2 rz,  depth = offset / dot,  z = fp32_rn(depth * rz)
+ * (n, offset: the layer's fp32 values widened).  The layer covers the pixel when z is finite and z > 0 (a plane
+ * behind the camera, an edge-on ray and a NaN plane cover nothing); a layer whose mask is outside [0, n_masks)
+ * covers nothing.  The covering layer of smallest z wins the pixel, the earlier one in the list on equal z:
+ *     depth_out [n_frames][H][W] fp32   the winner's z, 0.0f where no layer covers the pixel
+ *     rgb_out   [n_frames][H][W][3] u8  the winner's rgb, bg_rgb (HOST, 3 bytes) where none does
+ * Either output may be NULL (not written).  bits/bbox: the mask pool [n_masks][H][pitch] of the camera's H x W
+ * and its a3d_mask_meta boxes (bbox may be NULL: same output, no culling).  layers, layer_begin [n_frames + 1]
+ * DEVICE.  H, W <= A3D_RENDER_MAX_SIDE, any number of frames and layers.  One CTA per (frame, band of rows):
+ * the frame's layers whose box misses the band are culled first, in batches, and the band's running best
+ * (z, colour) stays in shared memory until its outputs are written once.                                  */
+int a3d_plane_maps(const a3d_camera_t* cam, int n_frames, const uint32_t* bits, const int32_t* bbox, int64_t n_masks,
+                   const a3d_plane_layer_t* layers, const int64_t* layer_begin, const uint8_t bg_rgb[3],
+                   float* depth_out, uint8_t* rgb_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
